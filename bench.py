@@ -8,6 +8,7 @@ NegBinom 1000 features, N=20, 256 particles, rho=0.25).
 
   python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
   python bench.py --impl reference ...                   # the restated reference on the host CPU
+  python bench.py ... --dump-outputs DIR                 # also write the last timed sweep's results as DIR/*.npy
 
 Prints ONE JSON line (contract in the task statement).  Besides the headline workload the line
 carries: `parity` (one sweep checked against the oracle before anything is timed - the oracle is
@@ -72,6 +73,25 @@ def make_workload(name, seed_shift=0, particles=None, **over):
 def dense_evals_per_sweep(cfg):
     steps = cfg["n"] - cfg["n1"] + 1
     return steps * cfg["P"] * cfg["N"] * sum(d.shape[1] for d in cfg["data"])
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res):
+    """Writes what a caller of the sweep receives (one download) as `out_dir/<name>.npy` in float64, so that two
+    builds run with the same arguments can be compared output for output.  An array larger than its share of
+    DUMP_BYTES is replaced by a fixed, seeded sample of its flattened elements."""
+    arrays = {k: np.asarray(v) for k, v in res.items() if isinstance(v, np.ndarray)}
+    arrays["p_star"] = np.array([res["p_star"]])
+    arrays["n_resamples"] = np.array([res["n_resamples"]])
+    share = DUMP_BYTES // len(arrays) // 8
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.astype(np.float64)
+        if a.size > share:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def common_config(cfg, burn):
@@ -169,6 +189,8 @@ def run_reference(args):
             burn.append(dt)
         elif it >= n_burn + args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r)
     total = float(np.sum(times))
     dense = dense_evals_per_sweep(cfg)
     val = dense * args.steps / total
@@ -294,8 +316,8 @@ class Runner:
         if self.world > 1:
             self.dist.barrier()
         torch.cuda.synchronize()
-        self.ctx.download()
-        return ev[0].elapsed_time(ev[steps]), [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)]
+        last = self.ctx.download()
+        return ev[0].elapsed_time(ev[steps]), [ev[i].elapsed_time(ev[i + 1]) for i in range(steps)], last
 
     def per_launch(self, steps, orders):
         """The same sweeps once more, one at a time: kernel time per launch (CUDA events inside the library,
@@ -468,8 +490,10 @@ def run_ours(args):
     run.chain(args.warmup, orders)   # warm-up = the SAME step as the timed one
     if rank == 0:
         sampler.mark()
-    dev_ms, step_ms = run.timed(args.steps, orders)
+    dev_ms, step_ms, last = run.timed(args.steps, orders)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     pl = run.per_launch(args.steps, orders)
     e2e_s = run.e2e(args.steps, orders)
     run.close()
@@ -553,7 +577,7 @@ def cfg4_block(world, rank, local, stream, flush, peak, peak_src, traffic_for, s
     run = Runner(cfg, world, rank, local, stream, flush)
     burn_ms = []
     run.chain(burn, orders, burn_ms)
-    dev_ms, step_ms = run.timed(steps, orders)
+    dev_ms, step_ms, _ = run.timed(steps, orders)
     pl = run.per_launch(steps, orders)
     run.close()
     k_ms = float(np.mean(pl["kms"]))
@@ -570,7 +594,7 @@ def cfg4_block(world, rank, local, stream, flush, peak, peak_src, traffic_for, s
         d.s, d.it = run.s, run.it   # the same chain state
         dsteps = 2
         d.chain(1, orders)
-        ddev, dstep = d.timed(dsteps, orders)
+        ddev, dstep, _ = d.timed(dsteps, orders)
         dpl = d.per_launch(dsteps + 1, orders)
         d.close()
         dk = float(np.mean(dpl["kms"]))
@@ -626,6 +650,8 @@ def main():
     ap.add_argument("--no-cfg4", action="store_true", help="skip the cfg4 block")
     ap.add_argument("--no-pmdi", action="store_true", help="skip the pmdi() end-to-end block")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity check against the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed sweep as DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
