@@ -212,13 +212,34 @@ int pmdi_cluster_eval(pmdi_ctx* ctx, int32_t k, const int64_t* rows, int64_t m, 
  *
  * (every cluster type of the reference has this form: feature-wise sufficient statistics, log-probability a sum
  * over features).  elem_kind: PMDI_F64 or PMDI_I64, the element type of the data the type is bound to.
- * Returns the type tag (>= 16) for pmdi_set_dataset.  The source is compiled (NVRTC, sm_100a) together with a
- * private copy of this library's kernels when a context first uses the type; a compile error is reported then,
- * with the compiler's log in pmdi_last_error().  One user type per context; single GPU; pool engine.
+ * Returns the type tag (>= 16) for pmdi_set_dataset; registering a name again replaces its source and keeps the tag.
+ *
+ * A context may bind a different user type to each of its K datasets (up to K <= 8 distinct types).  When it is
+ * first prepared, its user types are compiled (NVRTC, sm_100a) into ONE program together with a private copy of
+ * this library's set-up kernels and the sweep kernel of the context's engine; each source goes into a namespace of
+ * its own, so two types may both name their struct `Cluster`.  A compile error is reported then, with the
+ * compiler's log in pmdi_last_error().  WORDS sizes the type's statistics before anything is compiled: it is read
+ * from the source text (the number after the first "WORDS ... =") and the compiler checks it against the struct's
+ * constant; a source whose text says otherwise (a comment `// WORDS = 2` above the declaration) fails to compile
+ * with a message that names the type.
+ *   Engines: on one GPU a context with user types runs the pool engine unless PMDI_ENGINE=spec asks for the
+ *   speculative one; with the particles sharded the rule of the built-in types applies (spec for K <= 4, pool
+ *   above).  PMDI_ENGINE=pool / spec are honoured; the dense engine has no user hooks, PMDI_ENGINE=dense runs pool.
+ *   Compile time: about 10-20 s of CPU per program (the spec engine's is the larger).  Programs are cached per
+ *   process by engine and (struct name, element kind, source) of every type in slot order: another context with
+ *   the same types loads the cached one.  A type registered again with another source is recompiled for contexts
+ *   prepared afterwards; a context keeps the program it has.  PMDI_JIT_LOG set: one line per compile (with its
+ *   wall time) or cache hit on stderr.
+ *   Sharded particles: every rank registers its types in its own process (pmdi() does); pmdi_ipc_import rejects
+ *   ranks whose arena layouts - WORDS of the types included - disagree.
  */
 int pmdi_register_cluster_type(const char* name, const char* cuda_src, const char* struct_name, int32_t elem_kind,
                                int32_t* out_tag);
-/* Compiles a registered type now (no GPU needed) and reports the compiler's verdict; the log is in pmdi_last_error(). */
+/* Compiles a registered type now, alone in its program (no GPU needed), and reports the compiler's verdict; the log
+ * is in pmdi_last_error().  tag = PMDI_ALL_USER_TYPES: every type registered in this process, in registration order,
+ * in one program (at most 8).  The program is the pool engine's, or the spec engine's when PMDI_ENGINE=spec; it
+ * goes into the cache a context compiles through. */
+#define PMDI_ALL_USER_TYPES (-1)
 int pmdi_cluster_type_check(int32_t tag);
 
 /*

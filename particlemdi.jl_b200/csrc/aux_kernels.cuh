@@ -16,7 +16,7 @@ extern "C" __global__ void k_init_rows(DsDev ds, long long rows) {
     }
   } else if (ds.type == T_CATEGORICAL) {
     for (long long i = t0; i < rows * ds.Lmax * ds.Dp; i += stride) ds.cnt[i] = 0u;
-#ifdef PMDI_USER_STRUCT
+#ifdef PMDI_USER_TYPES
   } else if (ds.type == T_USER) {
     for (long long i = t0; i < rows * ds.Dp; i += stride) user_build_feature(ds, i / ds.Dp, (int)(i % ds.Dp), nullptr, 0, false);
 #endif
@@ -75,7 +75,7 @@ extern "C" __global__ void k_prefix_lists(SweepParams sp, int* members /* [K][n1
 __device__ __forceinline__ void build_row_feature(const DsDev& ds, const PoolDev* pd, long long row, int q,
                                                   const int* mem, int cnt, int use_flags) {
   const bool on = use_flags ? (ds.flag[q] != 0) : (q < ds.D);
-#ifdef PMDI_USER_STRUCT
+#ifdef PMDI_USER_TYPES
   if (ds.type == T_USER) { user_build_feature(ds, row, q, mem, cnt, on); return; }
 #endif
   if (ds.type == T_GAUSSIAN) {
@@ -190,17 +190,9 @@ extern "C" __global__ void k_logmarginal_part(DsDev ds, const int* c_off, const 
   const int cnt = c_off[c + 1] - c_off[c];
   const double n = (double)cnt;
   double lm;
-#ifdef PMDI_USER_STRUCT
+#ifdef PMDI_USER_TYPES
   if (ds.type == T_USER) {
-    double st[PmdiUser::WORDS];
-    PmdiUser::init(st);
-    if (on)
-      for (int t = 0; t < cnt; ++t) {
-        const double xv = ds.uW < 0 ? (double)((const int*)ds.x)[(size_t)mem[t] * ds.Dp + q]
-                                    : ((const double*)ds.x)[(size_t)mem[t] * ds.Dp + q];
-        PmdiUser::add(st, t + 1, xv);
-      }
-    lm = PmdiUser::logmarginal(st, cnt);
+    lm = user_logmarginal(ds, q, mem, cnt, on);
   } else
 #endif
   if (ds.type == T_GAUSSIAN) {
@@ -280,12 +272,12 @@ extern "C" __global__ void k_eval_row(SweepParams sp, int k, int obs, double* ou
   double acc = ds.rc[n];
   for (int j = 0; j < ds.J; ++j) {
     double v;
-#ifdef PMDI_USER_STRUCT
+#ifdef PMDI_USER_TYPES
     if (ds.type == T_USER) {
       const int fo = j * ds.FB + 2 * lane;
       const int nits = min(ds.FB / PMDI_WF, (ds.Dp - j * ds.FB) / PMDI_WF);
       double unused;
-      v = user_block(ds, ds.ust + (long long)row * PmdiUser::WORDS * ds.Dp + fo, 0, ds.flag + fo, nits, 0, n, 0u,
+      v = user_block(ds, ds.ust + row * user_row_words(ds) + fo, 0, ds.flag + fo, nits, 0, n, 0u,
                      (unsigned)__cvta_generic_to_shared(xs_raw) + fo * (ds.uW < 0 ? 4u : 8u), &unused);
     } else
 #endif

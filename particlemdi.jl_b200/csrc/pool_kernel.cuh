@@ -250,10 +250,11 @@ __device__ __noinline__ void pool_eval_rows(const SweepParams& sp, PoolSmem& sm,
             v = nb_block(ds.S + (long long)c * ds.Dp + fo, (long long)(d - c) * ds.Dp, ds.aux + (long long)c * ds.J + j,
                          ds.aux + (long long)d * ds.J + j, nit, mode, nc, xp + xo + fo * 4u, xc + xo + fo * 4u,
                          (unsigned)__cvta_generic_to_shared(T.lf), sp.lf_T, &vs);
-#ifdef PMDI_USER_STRUCT
+#ifdef PMDI_USER_TYPES
           } else if (ds.type == T_USER) {
             const unsigned eb = ds.uW < 0 ? 4u : 8u;
-            v = user_block(ds, ds.ust + (long long)c * PmdiUser::WORDS * ds.Dp + fo, (long long)(d - c) * PmdiUser::WORDS * ds.Dp,
+            const long long rw = user_row_words(ds);
+            v = user_block(ds, ds.ust + c * rw + fo, (d - c) * rw,
                            ds.flag + fo, nit, mode, nc, xp + xo + fo * eb, xc + xo + fo * eb, &vs);
 #endif
           } else {
@@ -656,6 +657,13 @@ __device__ __noinline__ void pool_row_pull(const SweepParams& sp, int k, long lo
 #pragma unroll 1
     for (long long q = 2 * lane; q < W; q += 64)
       *(ulonglong2*)(pd.cw + dst * W + q) = ldcg_u64x2(PMDI_SRC(pd.cw) + src * W + q);
+#ifdef PMDI_USER_TYPES
+  } else if (ds.type == T_USER) {  // ust[row][word][feature]: one contiguous range of |uW| * Dp doubles
+    const long long W = user_row_words(ds);
+#pragma unroll 1
+    for (long long q = 2 * lane; q < W; q += 64)
+      *(double2*)(ds.ust + dst * W + q) = ldcg_f64x2(PMDI_SRC(ds.ust) + src * W + q);
+#endif
   } else {
 #pragma unroll 1
     for (int q = 2 * lane; q < Dp; q += 64)
@@ -1002,6 +1010,8 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
   }                                                                                                       \
   __syncthreads();
 
+// (a run-time compiled program carries the sweep kernel of one engine only: PMDI_JIT_ENGINE 1 pool, 2 spec)
+#if !defined(PMDI_JIT_ENGINE) || PMDI_JIT_ENGINE == 1
 // production kernel: no debug capture, no tracing, no phase timing in the instruction stream
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool(const __grid_constant__ SweepParams sp_in) {
   POOL_KERNEL_PROLOGUE
@@ -1012,6 +1022,7 @@ extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool_dbg(const 
   POOL_KERNEL_PROLOGUE
   pool_sweep_body<true>(sp_s, sm, smem_raw, s_tmp);
 }
+#endif
 #undef TRACE
 
 // ------------------------------------------------------------------------------------------------

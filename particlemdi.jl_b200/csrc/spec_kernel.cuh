@@ -705,6 +705,13 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
             vd = nb_block(ds.S + (long long)v * ds.Dp + fo, (long long)(c - v) * ds.Dp, ds.aux + (long long)v * ds.J + jb,
                           ds.aux + (long long)c * ds.J + jb, nit, mode, nc, xp + xo + fo * 4u, xc + xo + fo * 4u,
                           (unsigned)__cvta_generic_to_shared(T.lf), sp.lf_T, &vs);
+#ifdef PMDI_USER_TYPES
+          } else if (ds.type == T_USER) {
+            const unsigned eb = ds.uW < 0 ? 4u : 8u;
+            const long long rw = user_row_words(ds);
+            vd = user_block(ds, ds.ust + v * rw + fo, (c - v) * rw, ds.flag + fo, nit, mode, nc, xp + xo + fo * eb,
+                            xc + xo + fo * eb, &vs);
+#endif
           } else {
             vd = cat_block(pd.cw + ((long long)v * ds.Dp + fo) * pd.wpf, (long long)(c - v) * ds.Dp * pd.wpf, pd.wpf,
                            pd.fpw, nit, mode, xp + xo + fo * 4u, xc + xo + fo * 4u, &vs);
@@ -778,7 +785,10 @@ __device__ __noinline__ void spec_row_pull(const SweepParams& sp, int4 j0, int4 
   const int4 i2 = ldcg_info(rinfo + (size_t)(parn ^ 1) * pd.cap + rb);     // step st+2: lp of the row
   const int4 i2c = ldcg_info(rinfo + (size_t)(parn ^ 1) * pd.cap + rc);    //            lp of its child
   const int n = ldcg_i32(PMDI_SRC(ds.n) + rb);
-  const long long W = ds.type == T_CATEGORICAL ? (long long)Dp * pd.wpf : (long long)Dp;  // 8-byte words per array of a row
+  long long W = ds.type == T_CATEGORICAL ? (long long)Dp * pd.wpf : (long long)Dp;  // 8-byte words per array of a row
+#ifdef PMDI_USER_TYPES
+  if (ds.type == T_USER) W = user_row_words(ds);
+#endif
   const long long per = ((W / 64 + SPEC_PULL_PARTS - 1) / SPEC_PULL_PARTS) * 64;
   const long long q_lo = part * per, q_hi = min(W, q_lo + per);
 #pragma unroll 1
@@ -796,6 +806,12 @@ __device__ __noinline__ void spec_row_pull(const SweepParams& sp, int4 j0, int4 
 #pragma unroll 1
       for (long long q = q_lo + 2 * lane; q < q_hi; q += 64)
         *(ulonglong2*)(pd.cw + dst * W + q) = ldcg_u64x2(PMDI_SRC(pd.cw) + src * W + q);
+#ifdef PMDI_USER_TYPES
+    } else if (ds.type == T_USER) {  // ust[row][word][feature]: one contiguous range of |uW| * Dp doubles
+#pragma unroll 1
+      for (long long q = q_lo + 2 * lane; q < q_hi; q += 64)
+        *(double2*)(ds.ust + dst * W + q) = ldcg_f64x2(PMDI_SRC(ds.ust) + src * W + q);
+#endif
     } else {
 #pragma unroll 1
       for (long long q = q_lo + 2 * lane; q < q_hi; q += 64)

@@ -762,6 +762,7 @@ __device__ __noinline__ bool do_resample(const SweepParams& sp, const CtaTables&
   return true;
 }
 
+#ifndef PMDI_USER_TYPES  // the dense engine has no user-type hooks: not part of a run-time compiled program
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep(const __grid_constant__ SweepParams sp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ __align__(16) SweepSmem sm;
@@ -1006,6 +1007,7 @@ extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep(const __grid_co
     for (int p = tid; p < sp.P; p += PMDI_NT) sp.lw_out[p] = sm.res_flag ? 1.0 : __ldcg(sp.lw + p);
   if (timing && tid < 8) sp.phase_ns[(size_t)cta * 8 + tid] = sm.tacc[tid] / NW;
   if (cta == 0 && tid == 0) sp.counters[2] = sm.ev;
+}
+#endif
 #undef PHASE_MARK
 #undef TRACE
-}

@@ -48,12 +48,27 @@ class NegBinomCluster:
 
 class UserCluster:
     """A user-defined cluster type (the reference's plugin contract, README.md:48-88): CUDA source of a struct with
-    init / logprob / add / logmarginal (include/pmdi_cuda.h, pmdi_register_cluster_type), compiled for the device
-    when a run first uses it.  ``integer_data``: the type is bound to Int64 data (counts, levels)."""
+    init / logprob / add / logmarginal (include/pmdi_cuda.h, pmdi_register_cluster_type).  ``integer_data``: the type
+    is bound to Int64 data (counts, levels).
+
+    Each dataset of a run may have a type of its own: ``pmdi([X_counts, X_expr], [MyPoisson, MyGaussian], ...)``.
+    The run compiles its user types into one program when it starts (about 10-20 s of CPU; cached for the rest of
+    the process, so a second run with the same types starts without compiling).  Each source lives in a namespace
+    of its own, so two types may both name their struct ``Cluster``.  One GPU runs the pool engine unless
+    ``PMDI_ENGINE=spec``; ``distributed=True`` shards the particles as for the built-in types.  The type is
+    registered in every process that reads ``tag`` (a rank started by torch.multiprocessing included), so the
+    object can be handed to the ranks of a distributed run as it is."""
 
     def __init__(self, name, cuda_src, struct_name=None, integer_data=False):
-        self.name = name
-        self.tag = capi.register_cluster_type(name, cuda_src, struct_name or name, capi.I64 if integer_data else capi.F64)
+        self.name, self.cuda_src = name, cuda_src
+        self.struct_name = struct_name or name
+        self.elem_kind = capi.I64 if integer_data else capi.F64
+        _ = self.tag  # registers now: a bad elem_kind or a missing library is reported here
+
+    @property
+    def tag(self):
+        """The type tag in this process (registering the same name and source again keeps it)."""
+        return capi.register_cluster_type(self.name, self.cuda_src, self.struct_name, self.elem_kind)
 
 
 def _tag(t):
