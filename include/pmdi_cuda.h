@@ -175,6 +175,36 @@ int pmdi_sweep_run(pmdi_ctx* ctx);                                   /* asynchro
 int pmdi_sweep_download(pmdi_ctx* ctx, pmdi_sweep_out* out);         /* sync + device -> host   */
 
 /*
+ * Groups: several independent contexts (chains) swept in ONE cooperative launch of the spec engine on one GPU.  A
+ * chain of the spec engine is bound by the latency of its per-observation steps and leaves most of the GPU idle; a
+ * group runs the members' grids side by side, each with its own barrier counter, so that several chains (other seeds,
+ * other N, other data) share the GPU instead of taking turns on it.  Results are those of each member swept alone.
+ *   pmdi_group_create  1..16 contexts, all on the same device, each on one GPU (not sharded), with built-in cluster
+ *                      types only and the spec engine (K <= 4, PMDI_ENGINE not pool / dense); a context is in at
+ *                      most one group.  Every member's datasets must be bound.  Each member gets a share of the SMs:
+ *                      the grid it has alone when the grids fit side by side, otherwise a share of the SM count in
+ *                      proportion to those grids (two 117-CTA members: 74 CTAs each).  Its role split and shared
+ *                      memory follow the share; a member whose share is too small for it (at least one proposal, one
+ *                      evaluation and the deciding CTA, and its tables in shared memory) makes the create fail with a
+ *                      message that names it, and nothing changes.
+ *   pmdi_group_run     after pmdi_sweep_upload on every member: each member's set-up kernels, one launch of the
+ *                      group kernel, each member's finish, all on the group's own stream (it waits for the members'
+ *                      uploads); then pmdi_sweep_download on each member as after pmdi_sweep_run.  A member's
+ *                      sweep_kernel_ms is the group kernel's time.  With PMDI_SWEEP_DEBUG on any member the
+ *                      instrumented twin runs; only the members that asked capture.  PMDI_TRACE_STEP is refused.
+ *   pmdi_group_destroy gives every member the whole GPU back.
+ * A member can still be swept alone (pmdi_sweep), on its share of the SMs; its barrier counters and step tags run on
+ * from sweep to sweep whether a sweep ran alone or in the group.  Creating or destroying a group re-sizes the members'
+ * grids: upload again before the next run.  pmdi_ctx_destroy of a member detaches it from its group (after any group
+ * launch in flight has finished); pmdi_group_run then fails until the group is destroyed.
+ */
+typedef struct pmdi_group pmdi_group;
+#define PMDI_GROUP_MAX_MEMBERS 16
+int pmdi_group_create(pmdi_group** out, pmdi_ctx* const* members, int32_t n_members);
+int pmdi_group_destroy(pmdi_group* group);
+int pmdi_group_run(pmdi_group* group);
+
+/*
  * Feature selection (src/pmdi.jl:120-128 and :354-370).
  * pmdi_feature_null: out[q] = -calc_logmarginal(all n_obs rows in one cluster)[q].
  * pmdi_feature_select: prob[q] = feature_null[q] + sum over occupied labels of

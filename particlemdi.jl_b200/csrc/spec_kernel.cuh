@@ -149,6 +149,16 @@ __device__ __noinline__ bool spec_xsync(const SweepParams& sp, SpecSmem& sm) {
   return true;
 }
 
+// This CTA's index within its context's grid.  A group launch (k_sweep_spec_group) runs the grids of several contexts
+// side by side in one cooperative grid; its prologue leaves each CTA's index within its own context's grid here.
+// (The trace and spec_xsync still read blockIdx.x: a group has no trace and no sharded member.)
+static __shared__ int spec_group_cta;
+template <bool GRP>
+__device__ __forceinline__ int spec_cta() {
+  if constexpr (GRP) return spec_group_cta;
+  else return (int)blockIdx.x;
+}
+
 __device__ __forceinline__ int4 ldcg_info(const RowInfo* p) { return __ldcg((const int4*)p); }
 __device__ __forceinline__ double info_lp(const int4& v) { return __hiloint2double(v.y, v.x); }
 
@@ -157,14 +167,14 @@ __device__ __forceinline__ double info_lp(const int4& v) { return __hiloint2doub
 // ------------------------------------------------------------------------------------------------
 // Proposal of one unit, read-only part (src/pmdi.jl:223-262): label, chosen row, its child, the
 // incremental weight - left in the unit tables.  One warp.
-template <bool DBG>
+template <bool DBG, bool GRP>
 __device__ __noinline__ void spec_propose(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int u, int step) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int K = sp.K, N = sp.N, P = sp.P, par = step & 1;
   const int ks = T.u_ks[u];
   const int k = ks & 0xff, sl = ks >> 8;
   const PoolDev& pd = sp.pd[k];
-  const int p = sp.slot0 + (int)blockIdx.x + sl * sp.GP;  // logical particle
+  const int p = sp.slot0 + spec_cta<GRP>() + sl * sp.GP;  // logical particle
   const int Npad = (N + 31) & ~31;
   double* lps = T.lp_s + warp * Npad;
   int* chs = T.ch_s + warp * Npad;
@@ -246,14 +256,14 @@ __device__ __noinline__ void spec_propose(const SweepParams& sp, SpecSmem& sm, c
 
 // Commit of one unit's proposal: the choice is counted, the label points at the child row, the
 // K-th commit of a particle folds its log-weight.  One warp (lane 0 works).
-template <bool DBG>
+template <bool DBG, bool GRP>
 __device__ __noinline__ void spec_commit(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int u, int step, int ns) {
   const int lane = threadIdx.x & 31;
   const int K = sp.K, N = sp.N, P = sp.P;
   const int ks = T.u_ks[u];
   const int k = ks & 0xff, sl = ks >> 8;
   const PoolDev& pd = sp.pd[k];
-  const int slot = (int)blockIdx.x + sl * sp.GP, p = sp.slot0 + slot;
+  const int slot = spec_cta<GRP>() + sl * sp.GP, p = sp.slot0 + slot;
   const int b3 = step % 3, z3 = (step + 1) % 3;  // choice counters: [3][cap], this step's and the next step's
   if (lane == 0) {
     const int c = T.u_c[u], label = T.lab_s[u], child = T.u_child[u];
@@ -423,12 +433,13 @@ __device__ __noinline__ bool spec_wait_decision(const SweepParams& sp, SpecSmem&
 }
 
 // (re)load the owned units' row maps into shared memory.  All threads of a P-CTA.
+template <bool GRP>
 __device__ __noinline__ void spec_load_units(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int ns) {
   const int K = sp.K, N = sp.N, nu = ns * K;
 #pragma unroll 1
   for (int i = threadIdx.x; i < nu * N; i += PMDI_NT) {
     const int u = i / N, m = i - u * N;
-    const int k = u % K, slot = (int)blockIdx.x + (u / K) * sp.GP;
+    const int k = u % K, slot = spec_cta<GRP>() + (u / K) * sp.GP;
     T.rm_s[i] = ldcg_i32(sp.pd[k].rowmap + ((size_t)(sm.ev & 1) * sp.Ps + slot) * N + m);
   }
 #pragma unroll 1
@@ -841,11 +852,12 @@ __device__ __noinline__ void spec_row_pull(const SweepParams& sp, int4 j0, int4 
 // st+1 were computed before the call and stay valid: a row's content does not depend on who refers
 // to it.
 // ------------------------------------------------------------------------------------------------
+template <bool GRP>
 __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int ns, int st,
                                            int* s_tmp, bool is_p, int e) {
   const int K = sp.K, N = sp.N, Ps = sp.Ps;
   const int ev = sm.ev;
-  const long long gt = (long long)blockIdx.x * PMDI_NT + threadIdx.x, GT = (long long)sp.G * PMDI_NT;
+  const long long gt = (long long)spec_cta<GRP>() * PMDI_NT + threadIdx.x, GT = (long long)sp.G * PMDI_NT;
   const int parn = (st + 1) & 1;  // info of step st+1: lp and child ids of everything that may be live;
                                   // also the copy of the reference counts the fix of step st+1 will read
   const bool has_next = st + 1 < sp.steps;
@@ -855,7 +867,7 @@ __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, 
 #define RS_MARK(i_) if (tm) { const unsigned long long n_ = globaltimer_ns(); sm.tacc[i_] += (n_ - t_) * POOL_NW; t_ = n_; }
   // every E-CTA (of every rank) has finished E'(st+2), every commit of step st is in
   if (!spec_xsync(sp, sm)) return false;
-  if ((int)blockIdx.x == sp.G - 1) {  // the D-CTA knows the maximum; its dynamic shared memory is free for the plan
+  if (spec_cta<GRP>() == sp.G - 1) {  // the D-CTA knows the maximum; its dynamic shared memory is free for the plan
     extern __shared__ __align__(16) unsigned char plan_raw[];  // (the dynamic shared memory, from its base)
     PlanScratch sc = {sp.sc_w, sp.sc_pp, sp.sc_u, sp.sc_j, sp.sc_anc0};
     if (sp.plan_smem) {
@@ -1031,7 +1043,7 @@ __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, 
   if (threadIdx.x == 0) { sm.ev = ev + 1; sm.res_flag = 0; }
   __syncthreads();
   if (is_p) {
-    spec_load_units(sp, sm, T, ns);
+    spec_load_units<GRP>(sp, sm, T, ns);
   } else if (e >= 0) {  // every E-CTA takes the whole new list; the cached free ids went back with the scan
     const int nl = ldcg_i32(sp.gcnt);
 #pragma unroll 1
@@ -1044,11 +1056,11 @@ __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, 
   return !sm.fail;
 }
 
-template <bool DBG>
+template <bool DBG, bool GRP>
 __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem& sm, unsigned char* smem_raw, int* s_tmp) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int NW = POOL_NW;
-  const int cta = blockIdx.x;
+  const int cta = spec_cta<GRP>();
   const int K = sp.K, N = sp.N, steps = sp.steps, GP = sp.GP;
   const bool is_p = cta < GP;
   const int e = cta - GP;
@@ -1099,7 +1111,7 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
     for (int sl = tid; sl < ns; sl += PMDI_NT) { T.lw_s[sl] = sp.lw_init; T.pcount[sl] = 0; }
 #pragma unroll 1
     for (int u = tid; u < nu; u += PMDI_NT) T.u_ks[u] = (u % K) | ((u / K) << 8);
-    spec_load_units(sp, sm, T, ns);
+    spec_load_units<GRP>(sp, sm, T, ns);
   } else if (cta != sp.G - 1) {
     if (tid == 0)
       for (int s = 0; s < sp.obs_ring; ++s) pool_issue_obs(sp, s, xring, sm.obs_bar);
@@ -1139,10 +1151,10 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
     if (is_p) {
       // ---- P(t): proposals (read-only), the decision on the resampling after step t-1, commit
 #pragma unroll 1
-      for (int u = warp; u < nu; u += NW) spec_propose<DBG>(sp, sm, T, u, t);
+      for (int u = warp; u < nu; u += NW) spec_propose<DBG, GRP>(sp, sm, T, u, t);
       STRACE(t, 49)
 #pragma unroll 1
-      for (int u = warp; u < nu; u += NW) spec_commit<DBG>(sp, sm, T, u, t, ns);
+      for (int u = warp; u < nu; u += NW) spec_commit<DBG, GRP>(sp, sm, T, u, t, ns);
       PHASE_MARK(2)
       if (t > 0) {
         // The step was committed without knowing whether step t-1 ends in a resampling: the decision (an exchange
@@ -1160,18 +1172,18 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
           }
 #pragma unroll 1
           for (int sl = tid; sl < ns; sl += PMDI_NT) T.lw_s[sl] = T.lw_prev[sl];
-          if (!spec_resample(sp, sm, T, ns, t - 1, s_tmp, true, e)) return;
+          if (!spec_resample<GRP>(sp, sm, T, ns, t - 1, s_tmp, true, e)) return;
           PHASE_MARK(6)
 #pragma unroll 1
-          for (int u = warp; u < nu; u += NW) spec_propose<DBG>(sp, sm, T, u, t);
+          for (int u = warp; u < nu; u += NW) spec_propose<DBG, GRP>(sp, sm, T, u, t);
 #pragma unroll 1
-          for (int u = warp; u < nu; u += NW) spec_commit<DBG>(sp, sm, T, u, t, ns);
+          for (int u = warp; u < nu; u += NW) spec_commit<DBG, GRP>(sp, sm, T, u, t, ns);
         }
       }
     } else if (is_d) {
       if (t > 0) {
         spec_decide(sp, sm, t - 1);
-        if (sm.res_flag && !spec_resample(sp, sm, T, ns, t - 1, s_tmp, false, -1)) return;
+        if (sm.res_flag && !spec_resample<GRP>(sp, sm, T, ns, t - 1, s_tmp, false, -1)) return;
       }
     } else {
       // ---- E side: outcome of step t-1, then the children of step t and the predictive of x[t+1]
@@ -1192,7 +1204,7 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
           if (!spec_wait_decision(sp, sm, t - 1)) return;
         } else if (sm.fail) return;
         if (sm.res_flag) {
-          if (!spec_resample(sp, sm, T, ns, t - 1, s_tmp, false, e)) return;
+          if (!spec_resample<GRP>(sp, sm, T, ns, t - 1, s_tmp, false, e)) return;
           PHASE_MARK(6)
         }
       }
@@ -1205,7 +1217,7 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   if (is_d) spec_decide(sp, sm, steps - 1);
   else { __syncthreads(); if (!spec_wait_decision(sp, sm, steps - 1)) return; }
   const int final_res = sm.res_flag;
-  if (final_res && !spec_resample(sp, sm, T, ns, steps - 1, s_tmp, is_p, is_d ? -1 : e)) return;
+  if (final_res && !spec_resample<GRP>(sp, sm, T, ns, steps - 1, s_tmp, is_p, is_d ? -1 : e)) return;
   if (tid < K) {
     atomicAdd(sp.rows_eval + tid, (unsigned long long)sm.rows_eval[tid]);
     atomicAdd(sp.rows_ref + tid, (unsigned long long)sm.rows_ref[tid]);
@@ -1235,14 +1247,52 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   }                                                                                                       \
   __syncthreads();
 
+#ifndef PMDI_SPEC_GROUP  // (the group module, spec_group.cu, carries the group kernels alone)
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec(const __grid_constant__ SweepParams sp_in) {
   SPEC_KERNEL_PROLOGUE
-  spec_sweep_body<false>(sp_s, sm, smem_raw, s_tmp);
+  spec_sweep_body<false, false>(sp_s, sm, smem_raw, s_tmp);
 }
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_dbg(const __grid_constant__ SweepParams sp_in) {
   SPEC_KERNEL_PROLOGUE
-  spec_sweep_body<true>(sp_s, sm, smem_raw, s_tmp);
+  spec_sweep_body<true, false>(sp_s, sm, smem_raw, s_tmp);
 }
+#endif
+
+// Several contexts (chains) in ONE cooperative launch: member m owns CTAs cta0[m] .. cta0[m+1]-1 and runs its own sweep
+// on them with a member-local CTA index.  A member's barrier counter, watchdog and error word are its own context's
+// memory (reached through its SweepParams), so the members synchronise independently of each other.
+#define PMDI_GROUP_MAX 16
+struct SpecGroupMap {
+  int n;
+  int cta0[PMDI_GROUP_MAX + 1];
+};
+#ifdef PMDI_SPEC_GROUP
+#define SPEC_GROUP_PROLOGUE                                                                               \
+  extern __shared__ __align__(16) unsigned char smem_raw[];                                               \
+  __shared__ __align__(16) SpecSmem sm;                                                                   \
+  __shared__ int s_tmp[4];                                                                                \
+  __shared__ __align__(16) SweepParams sp_s;                                                              \
+  {                                                                                                       \
+    int m = 0;                                                                                            \
+    _Pragma("unroll 1") while (m + 1 < map.n && (int)blockIdx.x >= map.cta0[m + 1]) ++m;                  \
+    if (threadIdx.x == 0) spec_group_cta = (int)blockIdx.x - map.cta0[m];                                 \
+    const int4* src = (const int4*)(sps + m);                                                             \
+    int4* dst = (int4*)&sp_s;                                                                             \
+    _Pragma("unroll 1") for (int i = threadIdx.x; i < (int)(sizeof(SweepParams) / 16); i += PMDI_NT) dst[i] = __ldg(src + i); \
+  }                                                                                                       \
+  __syncthreads();
+
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_group(const SweepParams* __restrict__ sps,
+                                                                           const __grid_constant__ SpecGroupMap map) {
+  SPEC_GROUP_PROLOGUE
+  spec_sweep_body<false, true>(sp_s, sm, smem_raw, s_tmp);
+}
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_group_dbg(const SweepParams* __restrict__ sps,
+                                                                               const __grid_constant__ SpecGroupMap map) {
+  SPEC_GROUP_PROLOGUE
+  spec_sweep_body<true, true>(sp_s, sm, smem_raw, s_tmp);
+}
+#endif
 #undef STRACE
 
 // Start of a sweep: the rho-prefix clusters (rows 0..N-1) are shared by all particles

@@ -462,12 +462,115 @@ def posterior_similarity(alloc):
 
 
 # ------------------------------------------------------------------ the entry point
+class _Chain:
+    """One chain of ``pmdi()``: its host RNG, hyper-parameters, allocations, context and output files, and the host
+    steps of an iteration around the sweep (src/pmdi.jl:164-185 before it, :354-383 after it)."""
+
+    def __init__(self, dataFiles, types, N, particles, rho, seed, factorised, stale_gamma_table, sstar_compat,
+                 device_reductions, device, rank, world):
+        K, n_obs = len(dataFiles), int(dataFiles[0].shape[0])
+        self.K, self.N, self.n_obs, self.n1, self.seed = K, N, n_obs, int(math.floor(rho * n_obs)), seed
+        self.stale_gamma_table, self.factorised = stale_gamma_table, factorised
+        self.sstar_compat, self.device_reductions = sstar_compat, device_reductions
+        self.rng = rng = np.random.default_rng(seed)
+        npairs = K * (K - 1) // 2
+        self.M = np.full(K, 2.0)                                          # :59
+        self.gamma = rng.gamma(1.0 / N, 1.0, (N, K)) + EPS                # :60
+        self.phi = rng.gamma(1.0, 0.2, npairs) if K > 1 else np.zeros(1)  # :61
+        self.s = np.stack([1 + rng.choice(N, size=n_obs, p=self.gamma[:, k] / self.gamma[:, k].sum())
+                           for k in range(K)], axis=1).astype(np.int64)   # :63-66
+        self.tables = FactorisedZ(N, K) if factorised else HyperTables(N, K)
+        if not factorised:
+            self.tables.refresh(self.gamma)
+        Z = update_Z(self.phi, self.tables, self.gamma)                   # :95
+        self.v = update_v(n_obs, Z, rng)                                  # :96
+        self.counts = self.agree = None  # first iteration: counted from the initial allocation
+        self.ctx = capi.Context(dataFiles, types, N, particles, device=device, rank=rank, n_ranks=world)  # raises without a GPU
+        self.stats = dict(sweep_device_ms=0.0, n_resamples=0, iterations=0)
+        self.out = self.ffile = self.flags = self.feature_null = None
+
+    def open(self, dataFiles, dataNames, outputFile, featureSelect_file):
+        K, rng = self.K, self.rng
+        if featureSelect_file is not None:                        # :106-128
+            self.flags = [rng.random(d.shape[1]) < 0.5 for d in dataFiles]
+            names = [f"{dataNames[k]}_d{d + 1}" for k in range(K) for d in range(dataFiles[k].shape[1])]
+            self.ffile = open(featureSelect_file, "w")
+            self.ffile.write(",".join(names) + "\n")
+            self.ffile.write(",".join("true" if f else "false" for fl in self.flags for f in fl) + "\n")
+            for k in range(K):
+                self.ctx.set_flags(k, self.flags[k].astype(np.uint8))
+            self.feature_null = [self.ctx.feature_null(k) for k in range(K)]
+        self.out = open(outputFile, "w")
+        self.out.write(csv_header(K, self.n_obs, dataNames) + "\n")  # :147-154
+
+    def sweep_args(self, it):
+        """The hyper-parameter updates of iteration `it` (:172-185); returns the sweep's arguments."""
+        K, N, rng, tables = self.K, self.N, self.rng, self.tables
+        order_obs = rng.permutation(self.n_obs) + 1                  # :172
+        update_M(self.M, self.gamma, K, N, rng)                      # :176
+        if not self.stale_gamma_table and not self.factorised:
+            tables.refresh(self.gamma)
+        update_gamma(self.gamma, self.phi, self.v, self.M, self.s, tables, rng, counts_all=self.counts)  # :177
+        Pi = self.gamma / self.gamma.sum(axis=0, keepdims=True)     # :179
+        if not self.stale_gamma_table and not self.factorised:
+            tables.refresh(self.gamma)
+        if K > 1:
+            update_phi(self.phi, self.v, self.s, tables, rng, agree_all=self.agree, gamma=self.gamma)  # :181-183
+        Z = update_Z(self.phi, tables, self.gamma)                   # :184
+        self.v = update_v(self.n_obs, Z, rng)                        # :185
+        return dict(s=self.s, order_obs=order_obs, n1=self.n1, Pi=Pi, phi=self.phi if K > 1 else None,
+                    logweight_init=0.0 if it == 1 else 1.0,          # :99, :372
+                    seed=self.seed, it=it, sstar_compat=self.sstar_compat)
+
+    def record(self, r, it, thin, t0):
+        """What iteration `it` does after its sweep `r`: feature selection, align_labels!, the CSV rows."""
+        K, N, rng = self.K, self.N, self.rng
+        self.s = s = np.array(r["s"], dtype=np.int64, order="C")
+        self.stats["sweep_device_ms"] += r["device_ms"]
+        self.stats["n_resamples"] += r["n_resamples"]
+        if self.ffile is not None:                                # :354-370
+            for k in range(K):
+                _, fl = self.ctx.feature_select(k, s[:, k], self.feature_null[k], seed=self.seed, it=it)
+                self.flags[k] = fl.astype(bool)
+                self.ctx.set_flags(k, fl)
+        # :375 - and the counts the next update_gamma! / update_Phi! read (update_hypers.jl:72,109-115),
+        # from the tables the sweep reduced on the device
+        if not self.device_reductions:
+            align_labels(s, self.phi, self.gamma, N, K, rng)
+            self.counts = self.agree = None
+        elif K > 1:
+            self.counts, self.agree = align_labels_tables(s, r["contingency"], self.phi, self.gamma, N, K, rng)
+        else:
+            self.counts, self.agree = np.array(r["label_counts"]), None
+        ll = time.perf_counter() - t0                             # :377 (cumulative seconds)
+        if it % thin == 0:                                        # :378-383
+            self.out.write(csv_row(self.M, self.phi, ll, s) + "\n")
+            if self.ffile is not None:
+                self.ffile.write(",".join("true" if f else "false" for fl in self.flags for f in fl) + "\n")
+        self.stats["iterations"] = it
+        self.stats["loop_s"] = ll
+
+    def close(self):
+        for f in (self.out, self.ffile):
+            if f is not None:
+                f.close()
+        if getattr(self, "ctx", None) is not None:
+            self.ctx.close()
+
+
 def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, featureSelect=None,
          dataNames=None, seed=0, device=0, stale_gamma_table=False, sstar_compat=False, factorised=None,
-         device_reductions=True, reference_literal=False, distributed=False):
+         device_reductions=True, reference_literal=False, distributed=False, chains=1):
     """``pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile; thin, featureSelect,
     dataNames)`` of src/pmdi.jl:36-40.  Side effect: the CSV file(s); returns a small dict of
-    timings and counters (the reference returns nothing)."""
+    timings and counters (the reference returns nothing).
+
+    ``chains=C > 1`` runs C independent chains side by side on one GPU: chain c is the run ``pmdi(..., seed=seed + c)``
+    would make alone (same CSV rows but the elapsed-seconds column), and ``outputFile`` (and ``featureSelect`` when
+    given) are sequences of C paths.  The chains' host steps run in lockstep, and each iteration sweeps all C chains in
+    ONE launch of the spec engine (``capi.Group``), each chain on a share of the SMs.  Returns a list of C dicts.
+    Needs K <= 4, the built-in cluster types and one GPU (not ``distributed``).  Whether it pays depends on the
+    problem: see DESIGN.md §13 for the measured aggregate rates against sweeping the chains one after another."""
     if reference_literal:  # the literal reference in one switch: never-refreshed gamma table, trajectories not permuted
         stale_gamma_table, sstar_compat, factorised = True, True, False
     t_entry = time.perf_counter()
@@ -490,25 +593,30 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
     assert n1 >= 1, "floor(ρ * n_obs) must be at least 1 (order_obs[n1:n_obs], src/pmdi.jl:209)"
 
     types = [_tag(t) for t in dataTypes]
-    rng = np.random.default_rng(seed)
-    npairs = K * (K - 1) // 2
-    M = np.full(K, 2.0)                                           # :59
-    gamma = rng.gamma(1.0 / N, 1.0, (N, K)) + EPS                 # :60
-    phi = rng.gamma(1.0, 0.2, npairs) if K > 1 else np.zeros(1)   # :61
-    s = np.stack([1 + rng.choice(N, size=n_obs, p=gamma[:, k] / gamma[:, k].sum())
-                  for k in range(K)], axis=1).astype(np.int64)    # :63-66
+    C = int(chains)
+    if C < 1:
+        raise ValueError("chains must be >= 1")
+    outputs, fsel = [outputFile], [featureSelect]
+    if C > 1:
+        if distributed:
+            raise ValueError("chains > 1 runs several chains on one GPU; distributed=True shards one chain's particles "
+                             "over the GPUs of a node: choose one")
+        if K > 4:
+            raise ValueError("chains > 1 sweeps the chains in one launch of the spec engine, which runs K <= 4 "
+                             "datasets (K > 4 runs the pool engine, which has no group launch)")
+        if any(t >= 16 for t in types):
+            raise ValueError("chains > 1: user-defined cluster types run their own compiled kernels, which have no "
+                             "group launch; run their chains one at a time")
+        outputs = list(outputFile)
+        fsel = list(featureSelect) if featureSelect is not None else [None] * C
+        if len(outputs) != C or len(fsel) != C:
+            raise ValueError(f"chains={C}: outputFile (and featureSelect when given) need {C} paths")
     # the N^K-row tables of :69-92 where they are small, the factorised sums (FactorisedZ) otherwise
     if factorised is None:
         factorised = N ** K > 200_000
     if factorised and stale_gamma_table:
         raise ValueError("stale_gamma_table needs the literal N^K tables")
-    tables = FactorisedZ(N, K) if factorised else HyperTables(N, K)
-    if not factorised:
-        tables.refresh(gamma)
-    Z = update_Z(phi, tables, gamma)                              # :95
-    v = update_v(n_obs, Z, rng)                                   # :96
 
-    counts = agree = None  # first iteration: counted from the initial allocation
     # distributed: one process per GPU of a node (torch.distributed initialised by the caller), the particles sharded
     # over the ranks; every rank runs this same loop with the same seed (identical hyper-parameters everywhere),
     # rank 0 writes the files
@@ -516,74 +624,40 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
     if distributed:
         import torch.distributed as dist
         rank, world = dist.get_rank(), dist.get_world_size()
-    ctx = capi.Context(dataFiles, types, N, particles, device=device, rank=rank, n_ranks=world)  # raises without a GPU
-    if world > 1:
-        ctx.connect()
-    if rank != 0:
-        outputFile, featureSelect_file = "/dev/null", ("/dev/null" if featureSelect is not None else None)
-    else:
-        featureSelect_file = featureSelect
-    stats_out = dict(sweep_device_ms=0.0, n_resamples=0, iterations=0)
-    ffile = None
+    chain_list, group = [], None
     try:
-        feature_null = None
-        if featureSelect is not None:                             # :106-128
-            flags = [rng.random(d.shape[1]) < 0.5 for d in dataFiles]
-            names = [f"{dataNames[k]}_d{d + 1}" for k in range(K) for d in range(dataFiles[k].shape[1])]
-            ffile = open(featureSelect_file, "w")
-            ffile.write(",".join(names) + "\n")
-            ffile.write(",".join("true" if f else "false" for fl in flags for f in fl) + "\n")
-            for k in range(K):
-                ctx.set_flags(k, flags[k].astype(np.uint8))
-            feature_null = [ctx.feature_null(k) for k in range(K)]
-        with open(outputFile, "w") as out:
-            out.write(csv_header(K, n_obs, dataNames) + "\n")     # :147-154
-            t0 = time.perf_counter()
-            stats_out["setup_s"] = t0 - t_entry   # data to the device, pool allocation (and a user type's compilation)
-            out.write(csv_row(M, phi, 0, s) + "\n")               # :158
-            for it in range(1, iter + 1):                         # :164
-                order_obs = rng.permutation(n_obs) + 1            # :172
-                update_M(M, gamma, K, N, rng)                     # :176
-                if not stale_gamma_table and not factorised:
-                    tables.refresh(gamma)
-                update_gamma(gamma, phi, v, M, s, tables, rng, counts_all=counts)    # :177
-                Pi = gamma / gamma.sum(axis=0, keepdims=True)     # :179
-                if not stale_gamma_table and not factorised:
-                    tables.refresh(gamma)
-                if K > 1:
-                    update_phi(phi, v, s, tables, rng, agree_all=agree, gamma=gamma)  # :181-183
-                Z = update_Z(phi, tables, gamma)                  # :184
-                v = update_v(n_obs, Z, rng)                       # :185
+        for c in range(C):
+            chain_list.append(_Chain(dataFiles, types, N, particles, rho, seed + c, factorised, stale_gamma_table,
+                                     sstar_compat, device_reductions, device, rank, world))
+        if world > 1:
+            chain_list[0].ctx.connect()
+        if rank != 0:
+            outputs, fsel = ["/dev/null"], ["/dev/null" if featureSelect is not None else None]
+        for ch, o, f in zip(chain_list, outputs, fsel):
+            ch.open(dataFiles, dataNames, o, f)
+        if C > 1:
+            group = capi.Group([ch.ctx for ch in chain_list])
+        t0 = time.perf_counter()
+        for ch in chain_list:
+            ch.stats["setup_s"] = t0 - t_entry  # data to the device, pool allocation (and a user type's compilation)
+            ch.out.write(csv_row(ch.M, ch.phi, 0, ch.s) + "\n")  # :158
+        for it in range(1, iter + 1):                             # :164
+            args = [ch.sweep_args(it) for ch in chain_list]
+            if group is not None:
+                for ch, a in zip(chain_list, args):
+                    ch.ctx.upload(**a)
+                group.run()
+                res = [ch.ctx.download(cluster_sizes=False) for ch in chain_list]
+            else:
+                ctx = chain_list[0].ctx
                 do_sweep = ctx.sweep_sharded if world > 1 else ctx.sweep
-                r = do_sweep(s, order_obs, n1, Pi, phi if K > 1 else None,
-                             logweight_init=0.0 if it == 1 else 1.0,   # :99, :372
-                             seed=seed, it=it, sstar_compat=sstar_compat, cluster_sizes=False)  # :188-350, :373
-                s = np.array(r["s"], dtype=np.int64, order="C")
-                stats_out["sweep_device_ms"] += r["device_ms"]
-                stats_out["n_resamples"] += r["n_resamples"]
-                if featureSelect is not None:                     # :354-370
-                    for k in range(K):
-                        _, fl = ctx.feature_select(k, s[:, k], feature_null[k], seed=seed, it=it)
-                        flags[k] = fl.astype(bool)
-                        ctx.set_flags(k, fl)
-                # :375 - and the counts the next update_gamma! / update_Phi! read (update_hypers.jl:72,109-115),
-                # from the tables the sweep reduced on the device
-                if not device_reductions:
-                    align_labels(s, phi, gamma, N, K, rng)
-                    counts = agree = None
-                elif K > 1:
-                    counts, agree = align_labels_tables(s, r["contingency"], phi, gamma, N, K, rng)
-                else:
-                    counts, agree = np.array(r["label_counts"]), None
-                ll = time.perf_counter() - t0                     # :377 (cumulative seconds)
-                if it % thin == 0:                                # :378-383
-                    out.write(csv_row(M, phi, ll, s) + "\n")
-                    if ffile is not None:
-                        ffile.write(",".join("true" if f else "false" for fl in flags for f in fl) + "\n")
-                stats_out["iterations"] = it
-                stats_out["loop_s"] = ll
+                res = [do_sweep(**args[0], cluster_sizes=False)]  # :188-350, :373
+            for ch, r in zip(chain_list, res):
+                ch.record(r, it, thin, t0)
     finally:
-        ctx.close()
-        if ffile is not None:
-            ffile.close()
-    return stats_out
+        if group is not None:
+            group.close()
+        for ch in chain_list:
+            ch.close()
+    stats = [ch.stats for ch in chain_list]
+    return stats if C > 1 else stats[0]
