@@ -73,6 +73,19 @@ int pmdi_ipc_export(pmdi_ctx* ctx, void* handle_out /* PMDI_IPC_HANDLE_BYTES */,
 int pmdi_ipc_import(pmdi_ctx* ctx, const void* handles /* n_ranks x PMDI_IPC_HANDLE_BYTES */,
                     const int64_t* arena_bytes /* n_ranks, may be NULL */);
 
+/*
+ * The engine of this context, ahead of PMDI_ENGINE and of the default rule (spec for K <= 4, pool above; pool for user
+ * types on one GPU).  PMDI_ENGINE_AUTO keeps that rule; the numbering is that of pmdi_sweep_out.engine.  An
+ * environment variable is process-wide: this lets one context (a member of a group, say) run the spec engine without
+ * changing the engine of every other context.  The dense engine is not offered here (PMDI_ENGINE=dense).  Valid only
+ * before the context is first prepared (its first upload, sweep, feature, cluster-eval or IPC export call): the
+ * memory layout depends on the engine, and a later call fails.
+ */
+#define PMDI_ENGINE_AUTO (-1)
+#define PMDI_ENGINE_POOL 1
+#define PMDI_ENGINE_SPEC 2
+int pmdi_ctx_set_engine(pmdi_ctx* ctx, int32_t engine);
+
 /* Use an externally owned cudaStream_t (e.g. the host framework's current stream). */
 int pmdi_ctx_set_stream(pmdi_ctx* ctx, void* cuda_stream);
 void* pmdi_ctx_get_stream(pmdi_ctx* ctx);
@@ -179,9 +192,14 @@ int pmdi_sweep_download(pmdi_ctx* ctx, pmdi_sweep_out* out);         /* sync + d
  * chain of the spec engine is bound by the latency of its per-observation steps and leaves most of the GPU idle; a
  * group runs the members' grids side by side, each with its own barrier counter, so that several chains (other seeds,
  * other N, other data) share the GPU instead of taking turns on it.  Results are those of each member swept alone.
- *   pmdi_group_create  1..16 contexts, all on the same device, each on one GPU (not sharded), with built-in cluster
- *                      types only and the spec engine (K <= 4, PMDI_ENGINE not pool / dense); a context is in at
- *                      most one group.  Every member's datasets must be bound.  Each member gets a share of the SMs:
+ *   pmdi_group_create  1..16 contexts, all on the same device, each on one GPU (not sharded) and on the spec engine
+ *                      (built-in types: K <= 4 and PMDI_ENGINE not pool / dense, or pmdi_ctx_set_engine; user types:
+ *                      pmdi_ctx_set_engine(ctx, PMDI_ENGINE_SPEC) or PMDI_ENGINE=spec, since their one-GPU default
+ *                      is pool); a context is in at most one group.  Members with user-defined cluster types must all
+ *                      have the same types in the same slot order (the types of their own compiled programs); members
+ *                      with built-in types only may join them.  Such a group runs the group kernels compiled at run time
+ *                      with those types (NVRTC, see pmdi_group_type_check); a group of built-in members runs the ones
+ *                      built into this library.  Every member's datasets must be bound.  Each member gets a share of the SMs:
  *                      the grid it has alone when the grids fit side by side, otherwise a share of the SM count in
  *                      proportion to those grids (two 117-CTA members: 74 CTAs each).  Its role split and shared
  *                      memory follow the share; a member whose share is too small for it (at least one proposal, one
@@ -192,7 +210,7 @@ int pmdi_sweep_download(pmdi_ctx* ctx, pmdi_sweep_out* out);         /* sync + d
  *                      uploads); then pmdi_sweep_download on each member as after pmdi_sweep_run.  A member's
  *                      sweep_kernel_ms is the group kernel's time.  With PMDI_SWEEP_DEBUG on any member the
  *                      instrumented twin runs; only the members that asked capture.  PMDI_TRACE_STEP is refused.
- *   pmdi_group_destroy gives every member the whole GPU back.
+ *   pmdi_group_destroy gives every member the whole GPU back (and unloads the group's compiled kernels).
  * A member can still be swept alone (pmdi_sweep), on its share of the SMs; its barrier counters and step tags run on
  * from sweep to sweep whether a sweep ran alone or in the group.  Creating or destroying a group re-sizes the members'
  * grids: upload again before the next run.  pmdi_ctx_destroy of a member detaches it from its group (after any group
@@ -203,6 +221,9 @@ typedef struct pmdi_group pmdi_group;
 int pmdi_group_create(pmdi_group** out, pmdi_ctx* const* members, int32_t n_members);
 int pmdi_group_destroy(pmdi_group* group);
 int pmdi_group_run(pmdi_group* group);
+/* Compiles the group kernels for these user types (tags of pmdi_register_cluster_type, 1..8, in slot order) now, with
+ * no GPU, into the cache pmdi_group_create compiles through; the log is in pmdi_last_error(). */
+int pmdi_group_type_check(const int32_t* tags, int32_t n);
 
 /*
  * Feature selection (src/pmdi.jl:120-128 and :354-370).
@@ -252,11 +273,13 @@ int pmdi_cluster_eval(pmdi_ctx* ctx, int32_t k, const int64_t* rows, int64_t m, 
  * from the source text (the number after the first "WORDS ... =") and the compiler checks it against the struct's
  * constant; a source whose text says otherwise (a comment `// WORDS = 2` above the declaration) fails to compile
  * with a message that names the type.
- *   Engines: on one GPU a context with user types runs the pool engine unless PMDI_ENGINE=spec asks for the
- *   speculative one; with the particles sharded the rule of the built-in types applies (spec for K <= 4, pool
- *   above).  PMDI_ENGINE=pool / spec are honoured; the dense engine has no user hooks, PMDI_ENGINE=dense runs pool.
+ *   Engines: on one GPU a context with user types runs the pool engine unless PMDI_ENGINE=spec or
+ *   pmdi_ctx_set_engine asks for the speculative one; with the particles sharded the rule of the built-in types applies
+ *   (spec for K <= 4, pool above).  PMDI_ENGINE=pool / spec are honoured; the dense engine has no user hooks,
+ *   PMDI_ENGINE=dense runs pool.  Contexts with user types on the spec engine can be swept together in a group
+ *   (pmdi_group_create): the group compiles a program of its own, the "spec-group" program, with the group kernels.
  *   Compile time: about 10-20 s of CPU per program (the spec engine's is the larger).  Programs are cached per
- *   process by engine and (struct name, element kind, source) of every type in slot order: another context with
+ *   process by kind (pool, spec, spec-group) and (struct name, element kind, source) of every type in slot order: another context with
  *   the same types loads the cached one.  A type registered again with another source is recompiled for contexts
  *   prepared afterwards; a context keeps the program it has.  PMDI_JIT_LOG set: one line per compile (with its
  *   wall time) or cache hit on stderr.

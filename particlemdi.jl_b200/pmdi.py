@@ -55,7 +55,7 @@ class UserCluster:
     The run compiles its user types into one program when it starts (about 10-20 s of CPU; cached for the rest of
     the process, so a second run with the same types starts without compiling).  Each source lives in a namespace
     of its own, so two types may both name their struct ``Cluster``.  One GPU runs the pool engine unless
-    ``PMDI_ENGINE=spec``; ``distributed=True`` shards the particles as for the built-in types.  The type is
+    ``PMDI_ENGINE=spec`` (``chains > 1`` runs the spec engine); ``distributed=True`` shards the particles as for the built-in types.  The type is
     registered in every process that reads ``tag`` (a rank started by torch.multiprocessing included), so the
     object can be handed to the ranks of a distributed run as it is."""
 
@@ -467,7 +467,7 @@ class _Chain:
     steps of an iteration around the sweep (src/pmdi.jl:164-185 before it, :354-383 after it)."""
 
     def __init__(self, dataFiles, types, N, particles, rho, seed, factorised, stale_gamma_table, sstar_compat,
-                 device_reductions, device, rank, world):
+                 device_reductions, device, rank, world, engine=None):
         K, n_obs = len(dataFiles), int(dataFiles[0].shape[0])
         self.K, self.N, self.n_obs, self.n1, self.seed = K, N, n_obs, int(math.floor(rho * n_obs)), seed
         self.stale_gamma_table, self.factorised = stale_gamma_table, factorised
@@ -485,7 +485,8 @@ class _Chain:
         Z = update_Z(self.phi, self.tables, self.gamma)                   # :95
         self.v = update_v(n_obs, Z, rng)                                  # :96
         self.counts = self.agree = None  # first iteration: counted from the initial allocation
-        self.ctx = capi.Context(dataFiles, types, N, particles, device=device, rank=rank, n_ranks=world)  # raises without a GPU
+        self.ctx = capi.Context(dataFiles, types, N, particles, device=device, rank=rank, n_ranks=world,
+                                engine=engine)  # raises without a GPU
         self.stats = dict(sweep_device_ms=0.0, n_resamples=0, iterations=0)
         self.out = self.ffile = self.flags = self.feature_null = None
 
@@ -569,8 +570,12 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
     would make alone (same CSV rows but the elapsed-seconds column), and ``outputFile`` (and ``featureSelect`` when
     given) are sequences of C paths.  The chains' host steps run in lockstep, and each iteration sweeps all C chains in
     ONE launch of the spec engine (``capi.Group``), each chain on a share of the SMs.  Returns a list of C dicts.
-    Needs K <= 4, the built-in cluster types and one GPU (not ``distributed``).  Whether it pays depends on the
-    problem: see DESIGN.md §13 for the measured aggregate rates against sweeping the chains one after another."""
+    Needs K <= 4 and one GPU (not ``distributed``).  User-defined cluster types (``UserCluster`` or tags) work too: their
+    chains run on the spec engine, so chain c writes what ``pmdi(..., seed=seed + c)`` writes alone with
+    ``PMDI_ENGINE=spec`` (a single chain with user types still runs the pool engine by default).  Whether it pays
+    depends on the problem: see DESIGN.md §13 for the measured aggregate rates against sweeping the chains one after
+    another, with built-in and with user types (cfg2 with two user types: 1.6x at C = 2, 3.7x at C = 8 over sequential
+    spec; a one-chain group measured 0.997x, and ``chains=1`` runs no group)."""
     if reference_literal:  # the literal reference in one switch: never-refreshed gamma table, trajectories not permuted
         stale_gamma_table, sstar_compat, factorised = True, True, False
     t_entry = time.perf_counter()
@@ -604,9 +609,6 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
         if K > 4:
             raise ValueError("chains > 1 sweeps the chains in one launch of the spec engine, which runs K <= 4 "
                              "datasets (K > 4 runs the pool engine, which has no group launch)")
-        if any(t >= 16 for t in types):
-            raise ValueError("chains > 1: user-defined cluster types run their own compiled kernels, which have no "
-                             "group launch; run their chains one at a time")
         outputs = list(outputFile)
         fsel = list(featureSelect) if featureSelect is not None else [None] * C
         if len(outputs) != C or len(fsel) != C:
@@ -624,11 +626,13 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
     if distributed:
         import torch.distributed as dist
         rank, world = dist.get_rank(), dist.get_world_size()
+    # a group runs the spec engine; user types default to pool on one GPU, so their chains ask for spec themselves
+    engine = "spec" if C > 1 and any(t >= 16 for t in types) else None
     chain_list, group = [], None
     try:
         for c in range(C):
             chain_list.append(_Chain(dataFiles, types, N, particles, rho, seed + c, factorised, stale_gamma_table,
-                                     sstar_compat, device_reductions, device, rank, world))
+                                     sstar_compat, device_reductions, device, rank, world, engine))
         if world > 1:
             chain_list[0].ctx.connect()
         if rank != 0:

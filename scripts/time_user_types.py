@@ -81,7 +81,7 @@ def nvrtc_log(fn):
         text = f.read()
     sys.stderr.write(text)
     return out, [(m.group(1), m.group(2), float(m.group(3)))
-                 for m in re.finditer(r"nvrtc compiled (.*) for the (\w+) engine in ([0-9.]+) s", text)]
+                 for m in re.finditer(r"nvrtc compiled (.*) for the ([\w-]+) engine in ([0-9.]+) s", text)]
 
 
 def summary(name, chain, dev, ker, wall, extra=None):
