@@ -362,3 +362,142 @@ extern "C" __global__ void k_mark_x(const int* x, const uint8_t* flag, int* xq, 
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride)
     xq[i] = flag[i % Dp] ? x[i] : skip;
 }
+
+// ------------------------------------------------------------------------------------------
+// after the sweep kernel (every engine)
+// ------------------------------------------------------------------------------------------
+
+// Particle selection (src/pmdi.jl:345-350), lineage back-trace, s[:] = sstar[p_star,:,:] (:373),
+// plus the reductions the host's update_hypers reads (src/update_hypers.jl:72,109-115): label counts
+// per (label, dataset) and, per dataset pair, the number of observations with equal labels.
+// One block.  The sums over the particles are sequential (same bits as the reference's cumsum), read
+// from shared memory; the lineage changes at the resampling events only, so it is walked over the
+// event list (a few entries) and every step looks its segment up.
+#define FIN_PW 4096
+#define FIN_EV 512
+extern "C" __global__ void k_finish_pool(SweepParams sp, int compat, long long* s_out, long long* p_star_out,
+                              int* cur_at, long long* label_counts, long long* pair_agree,
+                              long long* contingency) {
+  const int t = threadIdx.x, NT = blockDim.x, P = sp.P, K = sp.K, N = sp.N;
+  __shared__ double red[32];
+  __shared__ double w_s[FIN_PW];
+  __shared__ int ev_step[FIN_EV], ev_cur[FIN_EV + 1];
+  __shared__ int n_ev;
+  const bool in_smem = P <= FIN_PW;
+  double mx = -INFINITY;
+#pragma unroll 1
+  for (int p = t; p < P; p += NT) mx = fmax(mx, sp.lw_out[p]);
+  mx = warp_max(mx);
+  if ((t & 31) == 0) red[t >> 5] = mx;
+  if (t == 0) n_ev = 0;
+  __syncthreads();
+  mx = red[0];
+#pragma unroll 1
+  for (int i = 1; i < (NT >> 5); ++i) mx = fmax(mx, red[i]);
+#pragma unroll 1
+  for (int p = t; p < P; p += NT) {
+    const double w = exp(sp.lw_out[p] - mx);
+    if (in_smem) w_s[p] = w; else sp.sc_w[p] = w;
+  }
+  // steps that ended with a resampling, by event number (events are numbered in step order)
+#pragma unroll 1
+  for (int st = t; st < sp.steps; st += NT) {
+    const int ev = sp.ev_of_step[st];
+    if (ev >= 0) { atomicMax(&n_ev, ev + 1); if (ev < FIN_EV) ev_step[ev] = st; }
+  }
+  __syncthreads();
+  const int E = n_ev;
+  if (t == 0) {
+    const double* w = in_smem ? w_s : sp.sc_w;
+    double tot = 0.0;
+    for (int p = 0; p < P; ++p) tot += w[p];
+    const double u = sp.tape_select ? sp.tape_select[0] : pmdi_philox_uniform(sp.seed, sp.iter, DRAW_SELECT, 0, 0, 0);
+    const double thr = u * tot;
+    int i = 0;
+    double cw = w[0];
+    while (cw < thr && i < P - 1) { ++i; cw += w[i]; }
+    *p_star_out = i + 1;
+    // lineage of p_star through the resampling events, backwards (src/__pmdi.jl:285)
+    if (E <= FIN_EV) {
+      ev_cur[E] = i;
+      for (int e = E - 1; e >= 0; --e)
+        ev_cur[e] = compat ? i : sp.anc_log[(size_t)e * P + ev_cur[e + 1]] - 1;
+    } else {
+      int cur = i;
+      for (int st = sp.steps - 1; st >= 0; --st) {
+        const int ev = sp.ev_of_step[st];
+        if (ev >= 0 && !compat) cur = sp.anc_log[(size_t)ev * P + cur] - 1;
+        cur_at[st] = cur;
+      }
+    }
+  }
+#pragma unroll 1
+  for (size_t i = t; i < (size_t)K * sp.n_obs; i += NT) s_out[i] = sp.s_in[i];
+#pragma unroll 1
+  for (int i = t; i < N * K; i += NT) label_counts[i] = 0;
+#pragma unroll 1
+  for (int i = t; i < K * (K - 1) / 2; i += NT) pair_agree[i] = 0;
+#pragma unroll 1
+  for (int i = t; i < K * (K - 1) / 2 * N * N; i += NT) contingency[i] = 0;
+  __syncthreads();
+  if (E <= FIN_EV) {
+    // the particle a step's allocation is read from: the lineage after undoing every event at or
+    // after this step = entry of the first event whose step is >= st
+#pragma unroll 1
+    for (int st = t; st < sp.steps; st += NT) {
+      int lo = 0, hi = E;
+#pragma unroll 1
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (ev_step[mid] >= st) hi = mid; else lo = mid + 1; }
+      cur_at[st] = ev_cur[lo];
+    }
+    __syncthreads();
+  }
+#pragma unroll 1
+  for (int idx = t; idx < sp.steps * K; idx += NT) {
+    const int st = idx / K, k = idx - st * K;
+    const int obs = sp.order[sp.n1 - 1 + st];
+    s_out[(size_t)k * sp.n_obs + obs] = 1 + sp.alloc_log[((size_t)st * K + k) * P + cur_at[st]];
+  }
+  __syncthreads();
+#pragma unroll 1
+  for (size_t i = t; i < (size_t)K * sp.n_obs; i += NT)
+    atomicAdd((unsigned long long*)&label_counts[(i / sp.n_obs) * N + (s_out[i] - 1)], 1ull);
+#pragma unroll 1
+  for (int i = t; i < sp.n_obs; i += NT) {
+    int idx = 0;
+#pragma unroll 1
+    for (int k1 = 0; k1 < K - 1; ++k1)
+#pragma unroll 1
+      for (int k2 = k1 + 1; k2 < K; ++k2) {
+        const int la = (int)s_out[(size_t)k1 * sp.n_obs + i] - 1, lb = (int)s_out[(size_t)k2 * sp.n_obs + i] - 1;
+        if (la == lb) atomicAdd((unsigned long long*)&pair_agree[idx], 1ull);
+        atomicAdd((unsigned long long*)&contingency[((size_t)idx * N + lb) * N + la], 1ull);
+        ++idx;
+      }
+  }
+}
+
+// Sizes of the final particles' clusters (out.cluster_n): computed when the caller asks for them.
+extern "C" __global__ void k_cluster_n(SweepParams sp, long long* cluster_n) {
+  const int P = sp.P, K = sp.K, N = sp.N;
+  const int ev = (int)sp.counters[2];
+  const size_t stride = (size_t)gridDim.x * blockDim.x;
+#pragma unroll 1
+  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < (size_t)K * P * N; idx += stride) {
+    const int k = (int)(idx / ((size_t)P * N));
+    const size_t rem = idx - (size_t)k * P * N;
+    const int p = (int)(rem / N), m = (int)(rem % N);
+    long long v = -1;  // clusters of particles held by another rank: -1
+    if (sp.engine == 0) {
+      const int ls = sp.slot_of[(ev & 1) * P + p] - sp.slot0;
+      if (ls >= 0 && ls < sp.Ps) v = sp.ds[k].n[(long long)ls * N + m];
+    } else {
+      const int ls = p - sp.slot0;
+      if (ls >= 0 && ls < sp.Ps) {
+        const PoolDev& pd = sp.pd[k];
+        v = sp.ds[k].n[pd.rowmap[((size_t)(ev & 1) * sp.Ps + ls) * N + m]];
+      }
+    }
+    cluster_n[idx] = v;
+  }
+}

@@ -30,6 +30,7 @@ typedef unsigned long long uint64_t;
 #define PMDI_FB 256 /* features per work item (one warp, 4 iterations of 64) */
 #define PMDI_WF 64  /* features per warp iteration: 32 lanes x one 128-bit load */
 #define PMDI_NT 512 /* threads per CTA of the sweep kernel */
+#define PMDI_OBS_RING 4 /* observations in the sweep kernel's shared-memory ring (pool and spec: at most, as memory allows) */
 
 enum { T_GAUSSIAN = 0, T_CATEGORICAL = 1, T_NEGBINOM = 2, T_USER = 3 /* registered device functor */ };
 enum { DRAW_ALLOC = 0, DRAW_RESAMP = 1, DRAW_SHUFFLE = 2, DRAW_SELECT = 3, DRAW_FEATURE = 4 };

@@ -34,12 +34,14 @@
 // instruction cache per SM, a miss is an L2 round trip).  Hence: one block operator per cluster
 // type (pool_types.cuh), debug capture / tracing / phase timing compiled into a separate kernel
 // instantiation, the parameter block in shared memory, rare paths (resampling) out of line.
+//
+// The block operators are in pool_types.cuh; the observation ring, the resampling plan, the trace and the cross-rank
+// barrier, which the spec engine uses too, in sweep_common.cuh; the finish kernels in aux_kernels.cuh.
 #pragma once
 #include "pool_types.cuh"
-#include "sweep_kernel.cuh"
+#include "sweep_common.cuh"
 
 #define POOL_BIG_REF (1 << 30)
-#define POOL_NW (PMDI_NT / 32)
 #define POOL_FLAG_SHIFT 44  // grid counter: arrivals in the low 44 bits, resampling decisions above
 #define POOL_ARRIVE_MASK ((1ull << POOL_FLAG_SHIFT) - 1ull)
 
@@ -59,21 +61,8 @@ struct PoolSmem {
   int rbase[2][PMDI_MAX_K + 1];  // by step parity: first row task of each dataset
   unsigned rows_eval[PMDI_MAX_K], rows_ref[PMDI_MAX_K], rows_add[PMDI_MAX_K];
   unsigned long long tacc[8];
-  int tr_n[POOL_NW];
+  int tr_n[PMDI_NW];
 };
-
-// optional per-warp event trace of one CTA and one step (PMDI_TRACE_STEP): tag << 48 | clock64; stores only
-__device__ __forceinline__ void pool_trace(const SweepParams& sp, PoolSmem& sm, int step, unsigned tag) {
-  if (sp.trace && step == sp.trace_step && (int)blockIdx.x == sp.trace_cta && (threadIdx.x & 31) == 0) {
-    const int w = threadIdx.x >> 5;
-    const int n = ++sm.tr_n[w];
-    if (n < 128) {
-      sp.trace[w * 128 + n] = ((unsigned long long)tag << 48) | (clock64() & 0xFFFFFFFFFFFFull);
-      sp.trace[w * 128] = n;
-    }
-  }
-}
-#define TRACE(step_, tag_) if constexpr (DBG) pool_trace(sp, sm, (step_), (tag_));
 
 struct PoolTables {
   double* lf;      // [lf_T]
@@ -125,54 +114,9 @@ __device__ __noinline__ bool pool_gsync(const SweepParams& sp, PoolSmem& sm, int
   return sm.fail == 0;
 }
 
-// barrier over the CTAs of ALL ranks: local barrier, one arrival per rank on every rank's counter
-// (NVLink peer atomics), local barrier.  Resampling and the end of the sweep only.
+// barrier over the CTAs of ALL ranks (sweep_xsync)
 __device__ __noinline__ bool pool_xsync(const SweepParams& sp, PoolSmem& sm) {
-  if (!pool_gsync(sp, sm, 0, sp.R > 1)) return false;
-  if (sp.R > 1) {
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-      unsigned long long* xbar = (unsigned long long*)sp.bar + 1;
-      sm.xepoch += (unsigned long long)sp.R;
-      __threadfence_system();
-#pragma unroll 1
-      for (int r = 0; r < sp.R; ++r) atomicAdd_system(on_rank(sp, xbar, r), 1ull);
-      const unsigned long long t0 = globaltimer_ns();
-      unsigned spins = 0;
-#pragma unroll 1
-      while (ld_acquire_sys_u64(xbar) < sm.xepoch) {
-        if (((++spins) & 0x3ffu) == 0) {
-          if (__ldcg(sp.err) != 0) break;
-          if (globaltimer_ns() - t0 > sp.wd_ns) { atomicExch(sp.err, 77); break; }
-        }
-      }
-      __threadfence_system();
-    }
-    if (!pool_gsync(sp, sm)) return false;
-  }
-  return true;
-}
-
-// one thread: bulk-copy the K rows of the observation swept at `step` into its ring slot
-__device__ __noinline__ void pool_issue_obs(const SweepParams& sp, int step, unsigned char* xring,
-                                            unsigned long long* bars) {
-  if (step >= sp.steps) return;
-  const int b = step % sp.obs_ring;
-  const unsigned bar = (unsigned)__cvta_generic_to_shared(bars + b);
-  const int obs = sp.order[sp.n1 - 1 + step];
-  unsigned total = 0;
-#pragma unroll 1
-  for (int k = 0; k < sp.K; ++k) total += (unsigned)sp.ds[k].Dp * PMDI_XBYTES(sp.ds[k]);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // earlier generic reads of the slot
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(total) : "memory");
-#pragma unroll 1
-  for (int k = 0; k < sp.K; ++k) {
-    const DsDev& ds = sp.ds[k];
-    const unsigned bytes = (unsigned)ds.Dp * PMDI_XBYTES(ds);
-    const unsigned char* src = (const unsigned char*)ds.xstage + (size_t)obs * bytes;
-    const unsigned dst = (unsigned)__cvta_generic_to_shared(xring + (size_t)b * sp.sm_x_bytes + ds.x_off);
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-  }
+  return sweep_xsync(sp, sm, [&](bool sys) { return pool_gsync(sp, sm, 0, sys); });
 }
 
 // row tasks of the E phase of the step with parity b: the live rows as they are now (stable during
@@ -198,7 +142,7 @@ __device__ __noinline__ void pool_eval_rows(const SweepParams& sp, PoolSmem& sm,
                                             unsigned char* xring, int& obs_ok) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int b = st & 1, K = sp.K;
-  const int jq = sp.jq, rpc = POOL_NW / jq;
+  const int jq = sp.jq, rpc = PMDI_NW / jq;
   const int sub = warp / jq, wj = warp - sub * jq;
   const int total = sm.rbase[b][K];
   const unsigned xc = (unsigned)__cvta_generic_to_shared(xring + (size_t)(st % sp.obs_ring) * sp.sm_x_bytes);
@@ -419,7 +363,7 @@ __device__ __noinline__ void pool_propose(const SweepParams& sp, PoolSmem& sm, c
   double* lps = T.lp_s + warp * ((N + 31) & ~31);
   const int* rm = T.rm_s + u * N;
   const int empty = pd.cap - 1;
-  TRACE(step, 42)
+  SWEEP_TRACE(step, 42)
   // lp of the unit's N labels: one number per row (E phase); two labels per lane go out together
   double mx = -INFINITY;
   int occ = 0;
@@ -445,12 +389,12 @@ __device__ __noinline__ void pool_propose(const SweepParams& sp, PoolSmem& sm, c
                                  : pm_uniform(sp.seed, sp.iter, DRAW_ALLOC, step, k, p);
   mx = warp_max(mx);
   __syncwarp();
-  TRACE(step, 43)
+  SWEEP_TRACE(step, 43)
   // f = exp(lp - max) * Pi ; sequential cumsum over labels (src/pmdi.jl:236-241)
 #pragma unroll 1
   for (int m = lane; m < N; m += 32) lps[m] = pm_exp(lps[m] - mx) * T.Pi_s[k * N + m];
   __syncwarp();
-  TRACE(step, 44)
+  SWEEP_TRACE(step, 44)
   if (lane == 0) {
     double run = 0.0;
     int m = 0;
@@ -466,7 +410,7 @@ __device__ __noinline__ void pool_propose(const SweepParams& sp, PoolSmem& sm, c
     for (; m < N; ++m) { run += lps[m]; lps[m] = run; }
   }
   __syncwarp();
-  TRACE(step, 45)
+  SWEEP_TRACE(step, 45)
   const double tot = lps[N - 1];
   int label;
   if (p == 0) {
@@ -481,13 +425,13 @@ __device__ __noinline__ void pool_propose(const SweepParams& sp, PoolSmem& sm, c
       if (bb) { label = m0 + __ffs(bb) - 1; break; }
     }
   }
-  TRACE(step, 46)
+  SWEEP_TRACE(step, 46)
   int rank = 1;
   const int c = rm[label];
   if (lane == 0) rank = atomicAdd(pd.chosen + (size_t)par * pd.cap + c, 1);  // in flight during the log below
   const double inc = pm_log(tot) + mx;
   int last_particle = 0;
-  TRACE(step, 47)
+  SWEEP_TRACE(step, 47)
   if (lane == 0) {
     if (rank == 0) __stcg(pd.dst + (size_t)par * pd.cap + c, T.u_spare[u]);  // first chooser: the row a split would use
     T.u_c[u] = c; T.u_lab[u] = label; T.u_lead[u] = rank == 0;
@@ -529,94 +473,7 @@ __device__ __noinline__ void pool_propose(const SweepParams& sp, PoolSmem& sm, c
     __threadfence_block();
     pool_cta_partial(sp, T, ns, par);
   }
-  TRACE(step, 48)
-}
-
-// draw_partstar (src/misc.jl:27-47) by CTA 0, all threads: anc_log[ev][P] (1-based, non-decreasing,
-// anc[0] == 1).  The Fisher-Yates shuffle followed by partstar[1]=1 and sort! only decides WHICH
-// element of the sorted systematic sample the reference particle replaces: the one the shuffle
-// moves to position 1; that index is traced through the swaps without moving anything.
-// Scratch of the plan (P entries each): global memory, or the calling CTA's shared memory when it has room.
-struct PlanScratch { double *w, *pp, *u; int *j, *a0; };
-__device__ __noinline__ void pool_resample_plan(const SweepParams& sp, int step, int ev, double mx, int* s_tmp,
-                                                const double* lw, const PlanScratch sc) {
-  if (!lw) lw = sp.lw;  // (the spec engine keeps two copies of the log-weights, by step parity)
-  const int P = sp.P, t = threadIdx.x;
-#pragma unroll 1
-  for (int p = t; p < P; p += PMDI_NT) {
-    sc.w[p] = pm_exp(__ldcg(on_rank(sp, lw + p, p / sp.Ps)) - mx);  // the holder's copy (NVLink when remote)
-    const double us = sp.tape_shuffle ? sp.tape_shuffle[(size_t)step * P + p]
-                                      : pm_uniform(sp.seed, sp.iter, DRAW_SHUFFLE, step, 0, p);
-    int jj = 1 + (int)floor(us * (double)(p + 1));
-    if (jj > p + 1) jj = p + 1;
-    sc.j[p] = jj;
-  }
-  __syncthreads();
-  if (t == 0) {  // pprob = cumsum(exp.(logweight .- max)), sequential (misc.jl:29); loads sixteen ahead of the adds
-    double acc = 0.0;
-    int p = 0;
-#pragma unroll 1
-    for (; p + 16 <= P; p += 16) {
-      double v[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] = sc.w[p + i];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) { acc += v[i]; sc.pp[p + i] = acc; }
-    }
-#pragma unroll 1
-    for (; p < P; ++p) { acc += sc.w[p]; sc.pp[p] = acc; }
-  } else if (t == 32) {  // u, u + 1/P, ... by repeated addition (misc.jl:28,35)
-    const double r = sp.tape_resamp ? sp.tape_resamp[step] : pm_uniform(sp.seed, sp.iter, DRAW_RESAMP, step, 0, 0);
-    double u = r / (double)P;
-#pragma unroll 1
-    for (int i = 0; i < P; ++i) { sc.u[i] = u; u += 1.0 / (double)P; }
-  } else if (t == 64) {  // index of the pre-shuffle element that ends at position 1
-    int tt = 0, pos = 2;
-#pragma unroll 1
-    for (; pos + 15 <= P; pos += 16) {
-      int v[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) v[i] = sc.j[pos - 1 + i];
-#pragma unroll
-      for (int i = 0; i < 16; ++i)
-        if (v[i] - 1 == tt) tt = pos - 1 + i;
-    }
-#pragma unroll 1
-    for (; pos <= P; ++pos)
-      if (sc.j[pos - 1] - 1 == tt) tt = pos - 1;
-    s_tmp[0] = tt;
-  }
-  __syncthreads();
-  const double tot = sc.pp[P - 1];
-#pragma unroll 1
-  for (int i = t; i < P; i += PMDI_NT) {  // first p with pprob[p]/last >= u_i (misc.jl:33-38)
-    const double ui = sc.u[i];
-    int lo = 0, hi = P;
-#pragma unroll 1
-    while (lo < hi) {
-      const int mid = (lo + hi) >> 1;
-      if (pm_div(sc.pp[mid], tot) >= ui) hi = mid; else lo = mid + 1;
-    }
-    sc.a0[i] = (lo < P) ? lo + 1 : P;
-  }
-  __syncthreads();
-  const int drop = s_tmp[0];
-  int* anc = sp.anc_log + (size_t)ev * P;
-#pragma unroll 1
-  for (int i = t; i < P; i += PMDI_NT) {
-    const int a = (i == 0) ? 1 : ((i - 1 < drop) ? sc.a0[i - 1] : sc.a0[i]);
-    anc[i] = a;
-    if (sp.dbg_anc) sp.dbg_anc[(size_t)step * P + i] = a;
-  }
-  __syncthreads();
-  int dup = 0;  // particles that duplicate their predecessor's ancestor (a statistic)
-#pragma unroll 1
-  for (int i = 1 + t; i < P; i += PMDI_NT) dup += anc[i] == anc[i - 1];
-  if (dup) atomicAdd((unsigned long long*)&sp.counters[1], (unsigned long long)dup);
-  if (t == 0) {
-    sp.ev_of_step[step] = ev;
-    sp.counters[0] += 1;
-  }
+  SWEEP_TRACE(step, 48)
 }
 
 // (re)load the owned units' row maps into shared memory and reserve one row per unit.  All threads.
@@ -848,7 +705,7 @@ __device__ __noinline__ void pool_resolve_ranks(const SweepParams& sp, PoolSmem&
 template <bool DBG>
 __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem& sm, unsigned char* smem_raw, int* s_tmp) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int NW = POOL_NW;
+  const int NW = PMDI_NW;
   const int cta = blockIdx.x;
   const int K = sp.K, N = sp.N, steps = sp.steps, G = sp.G;
   const int Npad = (N + 31) & ~31;
@@ -886,7 +743,7 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
   for (int u = tid; u < nu; u += PMDI_NT) { T.u_duty[u] = 0; T.u_ks[u] = (u % K) | ((u / K) << 8); }
   if (tid < PMDI_MAX_K) { sm.rows_eval[tid] = 0; sm.rows_ref[tid] = 0; sm.rows_add[tid] = 0; }
   if (tid < 8) sm.tacc[tid] = 0;
-  if (tid < POOL_NW) sm.tr_n[tid] = 0;
+  if (tid < PMDI_NW) sm.tr_n[tid] = 0;
   if (tid == 0) {
     sm.res_flag = 0; sm.res_next = 0; sm.fail = 0; sm.ev = 0; sm.pdone = 0; sm.res_mx = 0.0;
     const unsigned long long b0 = __ldcg(sp.bar_state);  // the counters run on from the previous sweep
@@ -919,7 +776,7 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
 #pragma unroll 1
   for (int t = 0; t < steps; ++t) {
     const int par = t & 1;
-    TRACE(t, 40)
+    SWEEP_TRACE(t, 40)
     // ---- P(t): the last warp keeps house, the others propose
     if (t > 0) {
       if (tid == PMDI_NT - 1) pool_issue_obs(sp, t - 1 + sp.obs_ring, xring, sm.obs_bar);  // x[t-1] is dead: its slot refills
@@ -934,17 +791,17 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
       }
     }
     if (warp == NW - 1 && t + 1 < steps) pool_snapshot(sp, sm, par ^ 1);  // row tasks of E(t+1): the rows live now
-    TRACE(t, 41)
+    SWEEP_TRACE(t, 41)
 #pragma unroll 1
     for (int u = warp; u < nu; u += NW) pool_propose<DBG>(sp, sm, T, u, t, ns);
     PHASE_MARK(2)
-    TRACE(t, 49)
+    SWEEP_TRACE(t, 49)
     if (!pool_gsync(sp, sm)) return;  // B2(t): every choice, reservation and ESS partial is in
     PHASE_MARK(4)
-    TRACE(t, 50)
+    SWEEP_TRACE(t, 50)
     // ---- R(t)
     pool_resolve_units(sp, sm, T, nu, par);
-    TRACE(t, 51)
+    SWEEP_TRACE(t, 51)
     if (cta == 0 && warp == NW - 1) {
       if (sp.R > 1) {
         pool_push_rank_partial(sp, t);
@@ -960,11 +817,11 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
       }
     }
     PHASE_MARK(3)
-    TRACE(t, 52)
+    SWEEP_TRACE(t, 52)
     // ---- E(t+1)
     if (t + 1 < steps) pool_eval_rows(sp, sm, T, t + 1, par, xring, obs_ok);
     PHASE_MARK(1)
-    TRACE(t, 56)
+    SWEEP_TRACE(t, 56)
     if (!pool_gsync(sp, sm, sp.R == 1)) return;  // B1(t+1)
     PHASE_MARK(0)
   }
@@ -1010,8 +867,6 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
   }                                                                                                       \
   __syncthreads();
 
-// (a run-time compiled program carries the sweep kernel of one engine only: PMDI_JIT_ENGINE 1 pool, 2 spec)
-#if !defined(PMDI_JIT_ENGINE) || PMDI_JIT_ENGINE == 1
 // production kernel: no debug capture, no tracing, no phase timing in the instruction stream
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool(const __grid_constant__ SweepParams sp_in) {
   POOL_KERNEL_PROLOGUE
@@ -1022,19 +877,10 @@ extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool_dbg(const 
   POOL_KERNEL_PROLOGUE
   pool_sweep_body<true>(sp_s, sm, smem_raw, s_tmp);
 }
-#endif
-#undef TRACE
 
 // ------------------------------------------------------------------------------------------------
-// set-up and finish kernels of the pool engine
+// set-up kernel of the pool engine (the finish kernels, which every engine runs: aux_kernels.cuh)
 // ------------------------------------------------------------------------------------------------
-
-// all rows of a dataset's packed categorical counts to zero (the other statistics: k_init_rows)
-extern "C" __global__ void k_pool_init_rows(PoolDev pd, long long words) {
-  const long long stride = (long long)gridDim.x * blockDim.x;
-#pragma unroll 1
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < words; i += stride) pd.cw[i] = 0ull;
-}
 
 // Start of a sweep: the rho-prefix clusters (rows 0..N-1, built by k_prefix_build / k_proto_aux) are
 // shared by all particles (src/pmdi.jl:197-199: particle[u,:,k] .= id; clusters_counts = particles).
@@ -1071,162 +917,4 @@ extern "C" __global__ void k_pool_init(SweepParams sp) {
   for (int r = N + t; r < pd.cap - 1; r += NT) pd.freelist[nf0 + (r - N)] = r;
   __syncthreads();
   if (t == 0) { pd.refcnt[pd.cap - 1] = POOL_BIG_REF; ds.n[pd.cap - 1] = 0; }
-}
-
-// packed categorical counts of the prefix prototypes from the member lists (rows 0..N-1):
-// grid (ceil(Dp/128), N), thread per feature
-extern "C" __global__ void k_pool_prefix_cat(SweepParams sp, int k, const int* members, const int* off) {
-  const int m = blockIdx.y, q = blockIdx.x * blockDim.x + threadIdx.x;
-  const DsDev& ds = sp.ds[k];
-  const PoolDev& pd = sp.pd[k];
-  if (q >= ds.Dp) return;
-  const int b = off[k * (sp.N + 1) + m], e = off[k * (sp.N + 1) + m + 1];
-  const int* mem = members + (size_t)k * (sp.n1 - 1) + b;
-  unsigned long long* w = pd.cw + ((size_t)m * ds.Dp + q) * pd.wpf;
-#pragma unroll 1
-  for (int i = 0; i < pd.wpf; ++i) w[i] = 0ull;
-  if (ds.flag[q]) {
-    const int* x = (const int*)ds.x;
-    const int fw = 64 / pd.fpw;
-#pragma unroll 1
-    for (int t = 0; t < e - b; ++t) {
-      const int lv = x[(size_t)mem[t] * ds.Dp + q] - 1;
-      w[lv / pd.fpw] += 1ull << ((lv % pd.fpw) * fw);
-    }
-  }
-}
-
-// Particle selection (src/pmdi.jl:345-350), lineage back-trace, s[:] = sstar[p_star,:,:] (:373),
-// plus the reductions the host's update_hypers reads (src/update_hypers.jl:72,109-115): label counts
-// per (label, dataset) and, per dataset pair, the number of observations with equal labels.
-// One block.  The sums over the particles are sequential (same bits as the reference's cumsum), read
-// from shared memory; the lineage changes at the resampling events only, so it is walked over the
-// event list (a few entries) and every step looks its segment up.
-#define FIN_PW 4096
-#define FIN_EV 512
-extern "C" __global__ void k_finish_pool(SweepParams sp, int compat, long long* s_out, long long* p_star_out,
-                              int* cur_at, long long* label_counts, long long* pair_agree,
-                              long long* contingency) {
-  const int t = threadIdx.x, NT = blockDim.x, P = sp.P, K = sp.K, N = sp.N;
-  __shared__ double red[32];
-  __shared__ double w_s[FIN_PW];
-  __shared__ int ev_step[FIN_EV], ev_cur[FIN_EV + 1];
-  __shared__ int n_ev;
-  const bool in_smem = P <= FIN_PW;
-  double mx = -INFINITY;
-#pragma unroll 1
-  for (int p = t; p < P; p += NT) mx = fmax(mx, sp.lw_out[p]);
-  mx = warp_max(mx);
-  if ((t & 31) == 0) red[t >> 5] = mx;
-  if (t == 0) n_ev = 0;
-  __syncthreads();
-  mx = red[0];
-#pragma unroll 1
-  for (int i = 1; i < (NT >> 5); ++i) mx = fmax(mx, red[i]);
-#pragma unroll 1
-  for (int p = t; p < P; p += NT) {
-    const double w = exp(sp.lw_out[p] - mx);
-    if (in_smem) w_s[p] = w; else sp.sc_w[p] = w;
-  }
-  // steps that ended with a resampling, by event number (events are numbered in step order)
-#pragma unroll 1
-  for (int st = t; st < sp.steps; st += NT) {
-    const int ev = sp.ev_of_step[st];
-    if (ev >= 0) { atomicMax(&n_ev, ev + 1); if (ev < FIN_EV) ev_step[ev] = st; }
-  }
-  __syncthreads();
-  const int E = n_ev;
-  if (t == 0) {
-    const double* w = in_smem ? w_s : sp.sc_w;
-    double tot = 0.0;
-    for (int p = 0; p < P; ++p) tot += w[p];
-    const double u = sp.tape_select ? sp.tape_select[0] : pmdi_philox_uniform(sp.seed, sp.iter, DRAW_SELECT, 0, 0, 0);
-    const double thr = u * tot;
-    int i = 0;
-    double cw = w[0];
-    while (cw < thr && i < P - 1) { ++i; cw += w[i]; }
-    *p_star_out = i + 1;
-    // lineage of p_star through the resampling events, backwards (src/__pmdi.jl:285)
-    if (E <= FIN_EV) {
-      ev_cur[E] = i;
-      for (int e = E - 1; e >= 0; --e)
-        ev_cur[e] = compat ? i : sp.anc_log[(size_t)e * P + ev_cur[e + 1]] - 1;
-    } else {
-      int cur = i;
-      for (int st = sp.steps - 1; st >= 0; --st) {
-        const int ev = sp.ev_of_step[st];
-        if (ev >= 0 && !compat) cur = sp.anc_log[(size_t)ev * P + cur] - 1;
-        cur_at[st] = cur;
-      }
-    }
-  }
-#pragma unroll 1
-  for (size_t i = t; i < (size_t)K * sp.n_obs; i += NT) s_out[i] = sp.s_in[i];
-#pragma unroll 1
-  for (int i = t; i < N * K; i += NT) label_counts[i] = 0;
-#pragma unroll 1
-  for (int i = t; i < K * (K - 1) / 2; i += NT) pair_agree[i] = 0;
-#pragma unroll 1
-  for (int i = t; i < K * (K - 1) / 2 * N * N; i += NT) contingency[i] = 0;
-  __syncthreads();
-  if (E <= FIN_EV) {
-    // the particle a step's allocation is read from: the lineage after undoing every event at or
-    // after this step = entry of the first event whose step is >= st
-#pragma unroll 1
-    for (int st = t; st < sp.steps; st += NT) {
-      int lo = 0, hi = E;
-#pragma unroll 1
-      while (lo < hi) { const int mid = (lo + hi) >> 1; if (ev_step[mid] >= st) hi = mid; else lo = mid + 1; }
-      cur_at[st] = ev_cur[lo];
-    }
-    __syncthreads();
-  }
-#pragma unroll 1
-  for (int idx = t; idx < sp.steps * K; idx += NT) {
-    const int st = idx / K, k = idx - st * K;
-    const int obs = sp.order[sp.n1 - 1 + st];
-    s_out[(size_t)k * sp.n_obs + obs] = 1 + sp.alloc_log[((size_t)st * K + k) * P + cur_at[st]];
-  }
-  __syncthreads();
-#pragma unroll 1
-  for (size_t i = t; i < (size_t)K * sp.n_obs; i += NT)
-    atomicAdd((unsigned long long*)&label_counts[(i / sp.n_obs) * N + (s_out[i] - 1)], 1ull);
-#pragma unroll 1
-  for (int i = t; i < sp.n_obs; i += NT) {
-    int idx = 0;
-#pragma unroll 1
-    for (int k1 = 0; k1 < K - 1; ++k1)
-#pragma unroll 1
-      for (int k2 = k1 + 1; k2 < K; ++k2) {
-        const int la = (int)s_out[(size_t)k1 * sp.n_obs + i] - 1, lb = (int)s_out[(size_t)k2 * sp.n_obs + i] - 1;
-        if (la == lb) atomicAdd((unsigned long long*)&pair_agree[idx], 1ull);
-        atomicAdd((unsigned long long*)&contingency[((size_t)idx * N + lb) * N + la], 1ull);
-        ++idx;
-      }
-  }
-}
-
-// Sizes of the final particles' clusters (out.cluster_n): computed when the caller asks for them.
-extern "C" __global__ void k_cluster_n(SweepParams sp, long long* cluster_n) {
-  const int P = sp.P, K = sp.K, N = sp.N;
-  const int ev = (int)sp.counters[2];
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-#pragma unroll 1
-  for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < (size_t)K * P * N; idx += stride) {
-    const int k = (int)(idx / ((size_t)P * N));
-    const size_t rem = idx - (size_t)k * P * N;
-    const int p = (int)(rem / N), m = (int)(rem % N);
-    long long v = -1;  // clusters of particles held by another rank: -1
-    if (sp.engine == 0) {
-      const int ls = sp.slot_of[(ev & 1) * P + p] - sp.slot0;
-      if (ls >= 0 && ls < sp.Ps) v = sp.ds[k].n[(long long)ls * N + m];
-    } else {
-      const int ls = p - sp.slot0;
-      if (ls >= 0 && ls < sp.Ps) {
-        const PoolDev& pd = sp.pd[k];
-        v = sp.ds[k].n[pd.rowmap[((size_t)(ev & 1) * sp.Ps + ls) * N + m]];
-      }
-    }
-    cluster_n[idx] = v;
-  }
 }

@@ -35,8 +35,13 @@
 //   -- B(t) --
 // Same results as the two-barrier engine and as the dense form: a row's content and predictive
 // do not depend on who computes it or when.
+//
+// The pool's block operators come from pool_types.cuh; the observation ring, the resampling plan, the trace and the
+// cross-rank barrier from sweep_common.cuh; the finish kernels from aux_kernels.cuh.  With PMDI_SPEC_GROUP defined
+// this header compiles the group kernels and nothing else (spec_group.cu).
 #pragma once
-#include "pool_kernel.cuh"
+#include "pool_types.cuh"
+#include "sweep_common.cuh"
 
 #define SPEC_FC 256      // free-row ids per dataset cached by an E-CTA (shared memory)
 #define SPEC_EC 512      // entries of the live-row list kept in shared memory (the rest spills to HBM)
@@ -52,13 +57,13 @@ struct SpecSmem {
   int pdone;
   int lpar;                    // E-CTA: which copy of the entry list is current
   int cnt;                     // E-CTA: entries of the live-row list (all datasets)
-  int wsum[POOL_NW];           // E-CTA: per-warp survivor counts of the running fix
+  int wsum[PMDI_NW];           // E-CTA: per-warp survivor counts of the running fix
   int b_tt[PMDI_MAX_K], b_c[PMDI_MAX_K], b_cc[PMDI_MAX_K], b_next[PMDI_MAX_K];  // E-CTA: the empty clusters' children
   int kc[PMDI_MAX_K];          // E-CTA 0: entries per dataset
   unsigned kadd[PMDI_MAX_K];   // E-CTA 0: clusters that were chosen (the reference's cluster_add! calls)
   unsigned rows_eval[PMDI_MAX_K], rows_ref[PMDI_MAX_K], rows_spec[PMDI_MAX_K];
   unsigned long long tacc[8];
-  int tr_n[POOL_NW];
+  int tr_n[PMDI_NW];
 };
 
 struct SpecTables {
@@ -86,20 +91,9 @@ struct SpecTables {
   int* fc_top;     // [K]
 };
 
-#define STRACE(step_, tag_) if constexpr (DBG) spec_trace(sp, sm, (step_), (tag_));
 // bounds checks of the instrumented kernel instantiation (every debug-capture sweep of the parity tests runs them):
 // a row id outside its pool, a list longer than its storage or an id handed out twice ends the sweep with error 90+
 #define SCHECK(cond_, code_) if constexpr (DBG) { if (!(cond_)) { atomicExch(sp.err, (code_)); sm.fail = 1; } }
-__device__ __forceinline__ void spec_trace(const SweepParams& sp, SpecSmem& sm, int step, unsigned tag) {
-  if (sp.trace && step == sp.trace_step && (int)blockIdx.x == sp.trace_cta && (threadIdx.x & 31) == 0) {
-    const int w = threadIdx.x >> 5;
-    const int n = ++sm.tr_n[w];
-    if (n < 128) {
-      sp.trace[w * 128 + n] = ((unsigned long long)tag << 48) | (clock64() & 0xFFFFFFFFFFFFull);
-      sp.trace[w * 128] = n;
-    }
-  }
-}
 
 // grid barrier over this GPU's CTAs (both roles), all threads
 __device__ __noinline__ bool spec_gsync(const SweepParams& sp, SpecSmem& sm, bool sys = false) {
@@ -123,30 +117,9 @@ __device__ __noinline__ bool spec_gsync(const SweepParams& sp, SpecSmem& sm, boo
   return sm.fail == 0;
 }
 
-// barrier over the CTAs of ALL ranks: local barrier (peer stores made visible system-wide), one arrival per
-// rank on every rank's counter (NVLink peer atomics), local barrier.  Resampling and the end of the sweep.
+// barrier over the CTAs of ALL ranks (sweep_xsync)
 __device__ __noinline__ bool spec_xsync(const SweepParams& sp, SpecSmem& sm) {
-  if (!spec_gsync(sp, sm, sp.R > 1)) return false;
-  if (sp.R > 1) {
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-      unsigned long long* xbar = (unsigned long long*)sp.bar + 1;
-      sm.xepoch += (unsigned long long)sp.R;
-      __threadfence_system();
-#pragma unroll 1
-      for (int r = 0; r < sp.R; ++r) atomicAdd_system(on_rank(sp, xbar, r), 1ull);
-      const unsigned long long t0 = globaltimer_ns();
-      unsigned spins = 0;
-      while (ld_acquire_sys_u64(xbar) < sm.xepoch) {
-        if (((++spins) & 0x3ffu) == 0) {
-          if (__ldcg(sp.err) != 0) break;
-          if (globaltimer_ns() - t0 > sp.wd_ns) { atomicExch(sp.err, 77); break; }
-        }
-      }
-      __threadfence_system();
-    }
-    if (!spec_gsync(sp, sm)) return false;
-  }
-  return true;
+  return sweep_xsync(sp, sm, [&](bool sys) { return spec_gsync(sp, sm, sys); });
 }
 
 // This CTA's index within its context's grid.  A group launch (k_sweep_spec_group) runs the grids of several contexts
@@ -181,7 +154,7 @@ __device__ __noinline__ void spec_propose(const SweepParams& sp, SpecSmem& sm, c
   const int* rm = T.rm_s + u * N;
   const int empty = pd.cap - 1;
   const RowInfo* info = pd.info + (size_t)par * pd.cap;
-  STRACE(step, 42)
+  SWEEP_TRACE(step, 42)
   double mx = -INFINITY;
   int occ = 0;
 #pragma unroll 1
@@ -208,12 +181,12 @@ __device__ __noinline__ void spec_propose(const SweepParams& sp, SpecSmem& sm, c
                                  : pm_uniform(sp.seed, sp.iter, DRAW_ALLOC, step, k, p);
   mx = warp_max(mx);
   __syncwarp();
-  STRACE(step, 43)
+  SWEEP_TRACE(step, 43)
   // f = exp(lp - max) * Pi ; sequential cumsum over labels (src/pmdi.jl:236-241)
 #pragma unroll 1
   for (int m = lane; m < N; m += 32) lps[m] = pm_exp(lps[m] - mx) * T.Pi_s[k * N + m];
   __syncwarp();
-  STRACE(step, 44)
+  SWEEP_TRACE(step, 44)
   if (lane == 0) {
     double run = 0.0;
     int m = 0;
@@ -229,7 +202,7 @@ __device__ __noinline__ void spec_propose(const SweepParams& sp, SpecSmem& sm, c
     for (; m < N; ++m) { run += lps[m]; lps[m] = run; }
   }
   __syncwarp();
-  STRACE(step, 45)
+  SWEEP_TRACE(step, 45)
   const double tot = lps[N - 1];
   int label;
   if (p == 0) {
@@ -244,14 +217,14 @@ __device__ __noinline__ void spec_propose(const SweepParams& sp, SpecSmem& sm, c
       if (bb) { label = m0 + __ffs(bb) - 1; break; }
     }
   }
-  STRACE(step, 46)
+  SWEEP_TRACE(step, 46)
   const double inc = pm_log(tot) + mx;
   if (lane == 0) {
     T.u_c[u] = rm[label]; T.u_child[u] = chs[label]; T.u_occ[u] = occ;
     T.inc_s[u] = inc; T.lab_s[u] = label;
   }
   __syncwarp();
-  STRACE(step, 47)
+  SWEEP_TRACE(step, 47)
 }
 
 // Commit of one unit's proposal: the choice is counted, the label points at the child row, the
@@ -304,7 +277,7 @@ __device__ __noinline__ void spec_commit(const SweepParams& sp, SpecSmem& sm, co
       if (DBG && sp.dbg_lw) sp.dbg_lw[(size_t)step * P + p] = w;
     }
   }
-  STRACE(step, 48)
+  SWEEP_TRACE(step, 48)
 }
 
 // calc_ESS of step t (src/misc.jl:15-25, src/pmdi.jl:317) straight from the particles' log-weights (every
@@ -315,7 +288,7 @@ __device__ __noinline__ void spec_commit(const SweepParams& sp, SpecSmem& sm, co
 __device__ __noinline__ void spec_decide(const SweepParams& sp, SpecSmem& sm, int t) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, P = sp.P;
   // (with several ranks: this rank's particles; the ranks' partials are exchanged below)
-  const int per = (sp.Ps + POOL_NW - 1) / POOL_NW, p_lo = sp.slot0 + warp * per, p_hi = min(sp.slot0 + sp.Ps, p_lo + per);
+  const int per = (sp.Ps + PMDI_NW - 1) / PMDI_NW, p_lo = sp.slot0 + warp * per, p_hi = min(sp.slot0 + sp.Ps, p_lo + per);
   const double* lw = sp.lw + (size_t)(t & 1) * P;
   double mxv = -INFINITY;
 #pragma unroll 1
@@ -353,10 +326,10 @@ __device__ __noinline__ void spec_decide(const SweepParams& sp, SpecSmem& sm, in
   if (lane == 0) { sm.red[0][0][warp] = mxv; sm.red[0][0][16 + warp] = num; sm.red[0][0][32 + warp] = den; }
   __syncthreads();
   if (warp == 0) {
-    const double m = lane < POOL_NW ? sm.red[0][0][lane] : -INFINITY;
+    const double m = lane < PMDI_NW ? sm.red[0][0][lane] : -INFINITY;
     double mx = warp_max(m);
     double a = 0.0, b = 0.0;
-    if (lane < POOL_NW && m > -INFINITY) {
+    if (lane < PMDI_NW && m > -INFINITY) {
       const double e = pm_exp(m - mx);
       a = sm.red[0][0][16 + lane] * e;
       b = sm.red[0][0][32 + lane] * (e * e);
@@ -570,7 +543,7 @@ __device__ __noinline__ void spec_fix(const SweepParams& sp, SpecSmem& sm, const
     sm.b_next[tid] = in.z;
     sm.b_cc[tid] = in.w;
   }
-  STRACE(t1 + 1, 60)
+  SWEEP_TRACE(t1 + 1, 60)
   int nb = 0;  // entries of the new list so far (the same in every thread)
 #pragma unroll 1
   for (int base = 0; base < n_old; base += PMDI_NT) {
@@ -600,7 +573,7 @@ __device__ __noinline__ void spec_fix(const SweepParams& sp, SpecSmem& sm, const
         if (own) { __stcg(pd.refcnt + (size_t)parn * pd.cap + v, rf - tot); __stcg(pd.refcnt + (size_t)parn * pd.cap + c, tot); }
       }
     }
-    STRACE(t1 + 1, 61)
+    SWEEP_TRACE(t1 + 1, 61)
     // exclusive scan of the survivor counts over the CTA: list order is kept
     int incl = ns;
 #pragma unroll
@@ -620,7 +593,7 @@ __device__ __noinline__ void spec_fix(const SweepParams& sp, SpecSmem& sm, const
       __syncthreads();
       int wpre = 0, tot_all = 0;
 #pragma unroll
-      for (int w = 0; w < POOL_NW; ++w) {
+      for (int w = 0; w < PMDI_NW; ++w) {
         const int x = sm.wsum[w];
         if (w < warp) wpre += x;
         tot_all += x;
@@ -631,7 +604,7 @@ __device__ __noinline__ void spec_fix(const SweepParams& sp, SpecSmem& sm, const
       nb += tot_all;
       __syncthreads();
     }
-    STRACE(t1 + 1, 62)
+    SWEEP_TRACE(t1 + 1, 62)
   }
   if (n_old == 0) __syncthreads();  // b_* are complete
   else if (n_old <= 32) __syncwarp();  // ... written and read by the first warp
@@ -664,7 +637,7 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
                                        unsigned char* xring, int& obs_ok, int t_dec) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int K = sp.K, par = st & 1, GE = sp.G - sp.GP - 1;
-  const int jq = sp.jq, rpc = POOL_NW / jq;
+  const int jq = sp.jq, rpc = PMDI_NW / jq;
   const int sub = warp / jq, wj = warp - sub * jq;
   const int n_list = sm.cnt, total = n_list + K, lp = sm.lpar;
   const unsigned xc = (unsigned)__cvta_generic_to_shared(xring + (size_t)(st % sp.obs_ring) * sp.sm_x_bytes);
@@ -700,7 +673,7 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
         }
         const unsigned xo = (unsigned)ds.x_off;
         if (wj == 0 && lane < 2) rcv = __ldg(ds.rc + nc + 1 - lane);  // lane 1: the row's size constant, lane 0: its child's
-        STRACE(st - 1, 63)
+        SWEEP_TRACE(st - 1, 63)
 #pragma unroll 1
         for (int jb = wj; jb < ds.J; jb += jq) {
           const int q0 = jb * ds.FB;
@@ -735,9 +708,9 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
         }
       }
     }
-    STRACE(st - 1, 64)
+    SWEEP_TRACE(st - 1, 64)
     __syncthreads();
-    STRACE(st - 1, 65)
+    SWEEP_TRACE(st - 1, 65)
     if (active && wj == 0) {  // lane 1: the row, lane 0: its child - blocks in order, the size constant first
       const DsDev& ds = sp.ds[k];
       const PoolDev& pd = sp.pd[k];
@@ -759,7 +732,7 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
       }
       if (lane == 0) atomicAdd(&sm.rows_spec[k], mode ? 2u : 1u);
     }
-    STRACE(st - 1, 66)
+    SWEEP_TRACE(st - 1, 66)
   }
   // the decision on the resampling after step t_dec (published by the D-CTA early in this phase) is
   // fetched by a thread that has nothing to finish; the barrier below hands it to the CTA
@@ -864,7 +837,7 @@ __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, 
   // sub-phase timers (instrumented runs): tacc[4] wait for all CTAs + plan, [5] row maps + pulls, [7] recount + rebuild
   const bool tm = sp.phase_ns != nullptr && threadIdx.x == 0;
   unsigned long long t_ = tm ? globaltimer_ns() : 0ull;
-#define RS_MARK(i_) if (tm) { const unsigned long long n_ = globaltimer_ns(); sm.tacc[i_] += (n_ - t_) * POOL_NW; t_ = n_; }
+#define RS_MARK(i_) if (tm) { const unsigned long long n_ = globaltimer_ns(); sm.tacc[i_] += (n_ - t_) * PMDI_NW; t_ = n_; }
   // every E-CTA (of every rank) has finished E'(st+2), every commit of step st is in
   if (!spec_xsync(sp, sm)) return false;
   if (spec_cta<GRP>() == sp.G - 1) {  // the D-CTA knows the maximum; its dynamic shared memory is free for the plan
@@ -1059,7 +1032,7 @@ __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, 
 template <bool DBG, bool GRP>
 __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem& sm, unsigned char* smem_raw, int* s_tmp) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int NW = POOL_NW;
+  const int NW = PMDI_NW;
   const int cta = spec_cta<GRP>();
   const int K = sp.K, N = sp.N, steps = sp.steps, GP = sp.GP;
   const bool is_p = cta < GP;
@@ -1095,7 +1068,7 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   T.fc_top = T.fc_s + (size_t)K * SPEC_FC;
   if (tid < PMDI_MAX_K) { sm.rows_eval[tid] = 0; sm.rows_ref[tid] = 0; sm.rows_spec[tid] = 0; sm.kadd[tid] = 0; }
   if (tid < 8) sm.tacc[tid] = 0;
-  if (tid < POOL_NW) sm.tr_n[tid] = 0;
+  if (tid < PMDI_NW) sm.tr_n[tid] = 0;
   if (tid == 0) {
     sm.res_flag = 0; sm.fail = 0; sm.ev = 0; sm.pdone = 0; sm.res_mx = 0.0;
     sm.epoch = __ldcg(sp.bar_state); sm.xepoch = __ldcg(sp.bar_state + 1);  // the counters run on from the previous sweep
@@ -1147,12 +1120,12 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   PHASE_MARK(0)
 #pragma unroll 1
   for (int t = 0; t < steps; ++t) {
-    STRACE(t, 40)
+    SWEEP_TRACE(t, 40)
     if (is_p) {
       // ---- P(t): proposals (read-only), the decision on the resampling after step t-1, commit
 #pragma unroll 1
       for (int u = warp; u < nu; u += NW) spec_propose<DBG, GRP>(sp, sm, T, u, t);
-      STRACE(t, 49)
+      SWEEP_TRACE(t, 49)
 #pragma unroll 1
       for (int u = warp; u < nu; u += NW) spec_commit<DBG, GRP>(sp, sm, T, u, t, ns);
       PHASE_MARK(2)
@@ -1193,10 +1166,10 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
       // the distinct clusters the reference evaluates at step t (src/pmdi.jl:218-220): the list and the empty one
       if (e == 0 && tid < K) { sm.rows_eval[tid] += (unsigned)sm.kc[tid] + 1u; sm.kc[tid] = 0; }  // the next fix counts afresh
       PHASE_MARK(3)
-      STRACE(t, 51)
+      SWEEP_TRACE(t, 51)
       if (t + 1 < steps) spec_eval<DBG>(sp, sm, T, e, t + 1, xring, obs_ok, t - 1);
       PHASE_MARK(1)
-      STRACE(t, 52)
+      SWEEP_TRACE(t, 52)
       spec_refill(sp, sm, T);
       if (t > 0) {  // the decision on the resampling after step t-1: fetched inside the evaluation
         if (t + 1 >= steps) {
@@ -1209,7 +1182,7 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
         }
       }
     }
-    STRACE(t, 56)
+    SWEEP_TRACE(t, 56)
     if (!spec_gsync(sp, sm)) return;  // B(t)
     PHASE_MARK(0)
   }
@@ -1256,44 +1229,6 @@ extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_dbg(const 
   SPEC_KERNEL_PROLOGUE
   spec_sweep_body<true, false>(sp_s, sm, smem_raw, s_tmp);
 }
-#endif
-
-// Several contexts (chains) in ONE cooperative launch: member m owns CTAs cta0[m] .. cta0[m+1]-1 and runs its own sweep
-// on them with a member-local CTA index.  A member's barrier counter, watchdog and error word are its own context's
-// memory (reached through its SweepParams), so the members synchronise independently of each other.
-#define PMDI_GROUP_MAX 16
-struct SpecGroupMap {
-  int n;
-  int cta0[PMDI_GROUP_MAX + 1];
-};
-#ifdef PMDI_SPEC_GROUP
-#define SPEC_GROUP_PROLOGUE                                                                               \
-  extern __shared__ __align__(16) unsigned char smem_raw[];                                               \
-  __shared__ __align__(16) SpecSmem sm;                                                                   \
-  __shared__ int s_tmp[4];                                                                                \
-  __shared__ __align__(16) SweepParams sp_s;                                                              \
-  {                                                                                                       \
-    int m = 0;                                                                                            \
-    _Pragma("unroll 1") while (m + 1 < map.n && (int)blockIdx.x >= map.cta0[m + 1]) ++m;                  \
-    if (threadIdx.x == 0) spec_group_cta = (int)blockIdx.x - map.cta0[m];                                 \
-    const int4* src = (const int4*)(sps + m);                                                             \
-    int4* dst = (int4*)&sp_s;                                                                             \
-    _Pragma("unroll 1") for (int i = threadIdx.x; i < (int)(sizeof(SweepParams) / 16); i += PMDI_NT) dst[i] = __ldg(src + i); \
-  }                                                                                                       \
-  __syncthreads();
-
-extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_group(const SweepParams* __restrict__ sps,
-                                                                           const __grid_constant__ SpecGroupMap map) {
-  SPEC_GROUP_PROLOGUE
-  spec_sweep_body<false, true>(sp_s, sm, smem_raw, s_tmp);
-}
-extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_group_dbg(const SweepParams* __restrict__ sps,
-                                                                               const __grid_constant__ SpecGroupMap map) {
-  SPEC_GROUP_PROLOGUE
-  spec_sweep_body<true, true>(sp_s, sm, smem_raw, s_tmp);
-}
-#endif
-#undef STRACE
 
 // Start of a sweep: the rho-prefix clusters (rows 0..N-1) are shared by all particles
 // (src/pmdi.jl:197-199); the live ones open the list of live rows; every other row is free.
@@ -1333,3 +1268,40 @@ extern "C" __global__ void k_spec_init(SweepParams sp) {
   if (k == 0)
     for (int i = t; i < sp.steps; i += NT) sp.dec[i] = 0;
 }
+#endif
+
+// Several contexts (chains) in ONE cooperative launch: member m owns CTAs cta0[m] .. cta0[m+1]-1 and runs its own sweep
+// on them with a member-local CTA index.  A member's barrier counter, watchdog and error word are its own context's
+// memory (reached through its SweepParams), so the members synchronise independently of each other.
+#define PMDI_GROUP_MAX 16
+struct SpecGroupMap {
+  int n;
+  int cta0[PMDI_GROUP_MAX + 1];
+};
+#ifdef PMDI_SPEC_GROUP
+#define SPEC_GROUP_PROLOGUE                                                                               \
+  extern __shared__ __align__(16) unsigned char smem_raw[];                                               \
+  __shared__ __align__(16) SpecSmem sm;                                                                   \
+  __shared__ int s_tmp[4];                                                                                \
+  __shared__ __align__(16) SweepParams sp_s;                                                              \
+  {                                                                                                       \
+    int m = 0;                                                                                            \
+    _Pragma("unroll 1") while (m + 1 < map.n && (int)blockIdx.x >= map.cta0[m + 1]) ++m;                  \
+    if (threadIdx.x == 0) spec_group_cta = (int)blockIdx.x - map.cta0[m];                                 \
+    const int4* src = (const int4*)(sps + m);                                                             \
+    int4* dst = (int4*)&sp_s;                                                                             \
+    _Pragma("unroll 1") for (int i = threadIdx.x; i < (int)(sizeof(SweepParams) / 16); i += PMDI_NT) dst[i] = __ldg(src + i); \
+  }                                                                                                       \
+  __syncthreads();
+
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_group(const SweepParams* __restrict__ sps,
+                                                                           const __grid_constant__ SpecGroupMap map) {
+  SPEC_GROUP_PROLOGUE
+  spec_sweep_body<false, true>(sp_s, sm, smem_raw, s_tmp);
+}
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_group_dbg(const SweepParams* __restrict__ sps,
+                                                                               const __grid_constant__ SpecGroupMap map) {
+  SPEC_GROUP_PROLOGUE
+  spec_sweep_body<true, true>(sp_s, sm, smem_raw, s_tmp);
+}
+#endif

@@ -30,6 +30,7 @@
 // CTAs move the duplicated particles' rows (two blocking grid barriers), and the step restarts.
 #pragma once
 #include "cluster_types.cuh"
+#include "sweep_common.cuh"
 
 // exclusive scan of in[0..P) (global scratch, CTA-local use) into out; returns the total.
 __device__ int block_excl_scan(const int* in, int* out, int P, int* s_tmp /* PMDI_NT+1 ints */) {
@@ -156,7 +157,6 @@ __device__ __noinline__ void trace_mark(const SweepParams& sp, int step, unsigne
 }
 #define TRACE(step_, tag_) if (sp.trace) trace_mark(sp, (step_), (tag_));
 
-#define PMDI_OBS_RING 4
 #define PMDI_ITEM_FUSED 0x80000000u
 #define PMDI_ITEM_INVALID 0xFFFFFFFFu
 
@@ -210,25 +210,10 @@ struct CtaTables {
   int MU, cap;
 };
 
-__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
 // the grid counter as seen by this rank: other GPUs add to it through NVLink when R > 1
 __device__ __forceinline__ unsigned long long ld_counter(const SweepParams& sp) {
   const unsigned long long* bar = (const unsigned long long*)sp.bar;
   return sp.R > 1 ? ld_acquire_sys_u64(bar) : ld_acquire_u64(bar);
-}
-// the same object in rank r's shared arena (r == own rank: the pointer itself)
-template <class T>
-__device__ __forceinline__ T* on_rank(const SweepParams& sp, T* p, int r) {
-  return (T*)((char*)p + sp.peer_delta[r]);
 }
 // release everything this thread has observed, then add one arrival to EVERY rank's counter
 __device__ __forceinline__ void arrive_all(const SweepParams& sp) {
@@ -244,17 +229,6 @@ __device__ __forceinline__ void arrive_all(const SweepParams& sp) {
 __device__ __forceinline__ int ld_vol(const int* p) { return *(const volatile int*)p; }
 __device__ __forceinline__ void st_vol(int* p, int v) { *(volatile int*)p = v; }
 
-// ---- mbarrier / TMA bulk copy (observation ring) -----------------------------------------------
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count));
-}
-__device__ __forceinline__ bool mbar_try_wait(unsigned long long* bar, unsigned parity) {
-  unsigned ok;
-  asm volatile(
-      "{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-      : "=r"(ok) : "r"((unsigned)__cvta_generic_to_shared(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
 // one thread: bulk-copy the K rows of the observation swept at `step` into ring slot step % 4
 __device__ __noinline__ void issue_obs(const SweepParams& sp, int step, unsigned char* xring, unsigned long long* bars) {
   if (step >= sp.steps) return;
