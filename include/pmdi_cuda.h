@@ -306,6 +306,48 @@ int pmdi_psm_begin(pmdi_ctx* ctx);
 int pmdi_psm_add(pmdi_ctx* ctx, const int64_t* s);
 int pmdi_psm_get(pmdi_ctx* ctx, double* out);
 
+/*
+ * Posterior summaries of retained allocations, for one chain or several, with no sweep context: the reference's
+ * generate_psm (src/output_analysis/consensus_map.jl:31-65, per dataset and "Overall"), the least-squares consensus
+ * partition of Dahl (2006), and how far the chains' PSMs are apart.  The added samples stay on the device (n_obs * K
+ * bytes each), and the pair counts are kept as exact uint32 (about 2 * n_obs^2 * K * chains bytes).  DESIGN.md §14.
+ *   pmdi_summary_create     K datasets (1..8) of n_obs observations (1..65,535), labels 1..N (N <= 256), `chains`
+ *                           chains (1..64), on `device`.  Refuses, before allocating, a footprint that does not fit in
+ *                           the free device memory (counts, one chunk of samples per chain, one n_obs^2 read-out); the
+ *                           message states the bytes needed.
+ *   pmdi_summary_add        adds `rows` allocation matrices to chain `chain` (0-based), each n_obs x K column-major int64
+ *                           as pmdi_sweep takes them, one after another.  Every label must be in 1..N (checked first:
+ *                           a refused call adds nothing).  Copies through pinned staging on the summary's own stream and
+ *                           returns without waiting for the device; `s` may be reused at once.  Every 256 samples of a
+ *                           chain, and before any result below, the counts are brought up to date.  At most 2^24 rows in all.
+ *   pmdi_summary_rows       rows added to chain `chain` (-1 with the error in pmdi_last_error()).
+ *   pmdi_summary_psm        the full n_obs x n_obs PSM, row-major: count / rows (a true division of exact values, so it
+ *                           equals the same division done in f64 on the host bit for bit).  chain = -1 pools the chains
+ *                           (counts summed, divided by all rows); k = -1 is "Overall", (sum over k in order of PSM_k) / K.
+ *                           out is double, or float (the double result rounded) when as_f32 != 0.
+ *   pmdi_summary_ls         least-squares consensus of dataset k against the pooled PSM pi: for every sample r, in add
+ *                           order chain by chain, loss_out[r] = sum_{i<j} (delta_r(i,j) - pi_ij)^2 (computed exactly in
+ *                           integers, then rounded twice: to double, and in the division by rows^2).  best_chain / best_row: the lowest loss, the earliest sample
+ *                           on ties; partition_out: its n_obs labels 1..N.  Any output may be NULL.
+ *   pmdi_summary_agreement  chains >= 2: for every pair of chains a < b (row-major) and dataset k, out[pair * K + k] =
+ *                           max (max_out) and mean (mean_out) over i < j of |PSM_a(i,j) - PSM_b(i,j)|.
+ *   pmdi_summary_destroy    waits for the summary's work and frees everything.
+ */
+typedef struct pmdi_summary pmdi_summary;
+int pmdi_summary_create(pmdi_summary** out, int32_t device, int32_t K, int64_t n_obs, int32_t N, int32_t chains);
+int pmdi_summary_add(pmdi_summary* summary, int32_t chain, const int64_t* s, int64_t rows);
+int64_t pmdi_summary_rows(const pmdi_summary* summary, int32_t chain);
+int pmdi_summary_psm(pmdi_summary* summary, int32_t chain, int32_t k, void* out, int32_t as_f32);
+int pmdi_summary_ls(pmdi_summary* summary, int32_t k, double* loss_out, int32_t* best_chain, int64_t* best_row,
+                    int64_t* partition_out);
+int pmdi_summary_agreement(pmdi_summary* summary, double* max_out, double* mean_out);
+int pmdi_summary_destroy(pmdi_summary* summary);
+/* Host only (no device needed): the allocation columns of `rows` CSV rows of pmdi()'s output (header excluded), one
+ * row per line.  Each row's first `skip` columns are skipped, then `count` labels are read, written as integers
+ * ("12" or "12.0"), into out[row * count + column].  Anything else (a fractional label, too few or too many columns or
+ * rows) fails with the row and byte in pmdi_last_error(). */
+int pmdi_parse_allocations(const char* text, int64_t len, int64_t rows, int32_t skip, int64_t count, int64_t* out);
+
 /* The uniform the sweep uses for (kind, step, k, index); kinds as in the sweep:
    0 allocation, 1 resampling offset, 2 shuffle pick, 3 selection, 4 feature flag. */
 double pmdi_uniform(uint64_t seed, uint32_t iter, uint32_t kind, uint32_t step, uint32_t k,

@@ -22,6 +22,7 @@ There is no CPU fallback: without the CUDA library or a device this raises.
 from __future__ import annotations
 
 import math
+import os
 import time
 
 import numpy as np
@@ -449,6 +450,94 @@ def read_allocations(outputFile, K, n_obs, burnin=0, thin=1):
     return raw.reshape(raw.shape[0], K, n_obs).transpose(0, 2, 1).astype(np.int64)
 
 
+def _header_layout(header):
+    """(K, n_obs, dataNames) from the header ``csv_header`` writes."""
+    cols = header.strip().split(",")
+    K = sum(c.startswith("MassParameter_") for c in cols)
+    if K < 1 or "ll" not in cols:
+        raise ValueError("not a pmdi() output header (no MassParameter_k / ll columns)")
+    alloc = cols[n_hyper_columns(K):]
+    names = list(dict.fromkeys(c.rsplit("_n", 1)[0] for c in alloc))
+    if len(names) != K or len(alloc) % K:
+        raise ValueError(f"header has {K} mass parameters but allocation columns of {len(names)} datasets")
+    return K, len(alloc) // K, names
+
+
+def read_chains(outputFiles, burnin=0, thin=1):
+    """Allocations of one ``pmdi()`` CSV file or several (chains), with K, n_obs and the dataset names taken from the
+    header.  Returns (list of (rows, n_obs, K) int64 arrays, one per file, each what ``read_allocations(file, K, n_obs,
+    burnin, thin)`` returns; dataNames).  Every file must have the same layout.  Only the retained rows are parsed, and
+    their label columns are read as integers in C (``pmdi_parse_allocations``, no device needed); DESIGN.md §14 gives
+    its cost per row against ``np.loadtxt``."""
+    files = [outputFiles] if isinstance(outputFiles, (str, os.PathLike)) else list(outputFiles)
+    if not files:
+        raise ValueError("no output files")
+    if burnin < 0 or thin < 1:
+        raise ValueError("need burnin >= 0 and thin >= 1")
+    out, layout = [], None
+    for f in files:
+        with open(f, "rb") as fh:
+            header = fh.readline().decode()
+            body = fh.read()
+        lay = _header_layout(header)
+        if layout is not None and lay[:2] != layout[:2]:
+            raise ValueError(f"{f}: K, n_obs = {lay[:2]} differ from {layout[:2]} of {files[0]}")
+        layout = layout or lay
+        K, n_obs, _ = lay
+        total = body.count(b"\n") + (1 if body and not body.endswith(b"\n") else 0)
+        if thin == 1:  # the rows after the burn-in are one stretch of the text: no split into lines
+            at = 0
+            for _ in range(min(burnin, total)):
+                at = body.index(b"\n", at) + 1
+            text, rows = body[at:], max(total - burnin, 0)
+        else:
+            kept = body.split(b"\n")[:total][burnin::thin]
+            text, rows = b"\n".join(kept), len(kept)
+        try:
+            a = capi.parse_allocations(text, rows, n_hyper_columns(K), K * n_obs)
+        except ValueError as e:
+            raise ValueError(f"{f} (rows from {burnin + 1} every {thin}): {e}") from None
+        out.append(a.reshape(rows, K, n_obs).transpose(0, 2, 1))
+    return out, layout[2]
+
+
+def _summary_of(outputFiles, burnin, thin, device):
+    chains, _ = read_chains(outputFiles, burnin, thin)
+    rows, n_obs, K = chains[0].shape
+    if any(c.shape[0] == 0 for c in chains):
+        raise ValueError("a chain keeps no rows after burnin / thin")
+    N = int(max(c.max() for c in chains))
+    if N > 256:
+        raise ValueError(f"labels up to {N}: the summaries take at most 256")
+    S = capi.PosteriorSummary(K, n_obs, N, chains=len(chains), device=device)
+    for c, a in enumerate(chains):
+        S.add(c, a)
+    return S
+
+
+def generate_psm(outputFiles, burnin=0, thin=1, device=0):
+    """The reference's ``generate_psm(outputFile, burnin, thin)`` (consensus_map.jl:31-65) on the GPU, over one
+    CSV file or the files of several chains, pooled: shape (K + 1, n_obs, n_obs), the datasets in order, then Overall
+    (their sum in k order divided by K).  Each dataset's PSM equals ``posterior_similarity`` of the rows of all files
+    concatenated, bit for bit."""
+    with _summary_of(outputFiles, burnin, thin, device) as S:
+        return np.stack([S.psm(k) for k in range(S.K)] + [S.psm(None)])
+
+
+def consensus_partition(outputFiles, burnin=0, thin=1, device=0):
+    """Least-squares consensus (Dahl 2006) per dataset over the retained rows of one CSV file or several: the sample
+    closest to the pooled PSM.  Returns (n_obs, K) labels."""
+    with _summary_of(outputFiles, burnin, thin, device) as S:
+        return np.stack([S.least_squares(k)[0] for k in range(S.K)], axis=1)
+
+
+def chain_agreement(outputFiles, burnin=0, thin=1, device=0):
+    """(max, mean) over i < j of |PSM_a - PSM_b| for every pair of chains (files) a < b, row-major, and dataset:
+    two arrays of shape (C (C - 1) / 2, K)."""
+    with _summary_of(outputFiles, burnin, thin, device) as S:
+        return S.agreement()
+
+
 def posterior_similarity(alloc):
     """PSM per dataset (consensus_map.jl:50-56): fraction of retained rows in which two
     observations share a label.  Returns (K, n, n)."""
@@ -489,6 +578,7 @@ class _Chain:
                                 engine=engine)  # raises without a GPU
         self.stats = dict(sweep_device_ms=0.0, n_resamples=0, iterations=0)
         self.out = self.ffile = self.flags = self.feature_null = None
+        self.offer = None  # pmdi(summary=S): every CSV row's allocations go to S as well
 
     def open(self, dataFiles, dataNames, outputFile, featureSelect_file):
         K, rng = self.K, self.rng
@@ -546,6 +636,8 @@ class _Chain:
         ll = time.perf_counter() - t0                             # :377 (cumulative seconds)
         if it % thin == 0:                                        # :378-383
             self.out.write(csv_row(self.M, self.phi, ll, s) + "\n")
+            if self.offer is not None:
+                self.offer(s)
             if self.ffile is not None:
                 self.ffile.write(",".join("true" if f else "false" for fl in self.flags for f in fl) + "\n")
         self.stats["iterations"] = it
@@ -561,7 +653,7 @@ class _Chain:
 
 def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, featureSelect=None,
          dataNames=None, seed=0, device=0, stale_gamma_table=False, sstar_compat=False, factorised=None,
-         device_reductions=True, reference_literal=False, distributed=False, chains=1):
+         device_reductions=True, reference_literal=False, distributed=False, chains=1, summary=None):
     """``pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile; thin, featureSelect,
     dataNames)`` of src/pmdi.jl:36-40.  Side effect: the CSV file(s); returns a small dict of
     timings and counters (the reference returns nothing).
@@ -575,7 +667,12 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
     ``PMDI_ENGINE=spec`` (a single chain with user types still runs the pool engine by default).  Whether it pays
     depends on the problem: see DESIGN.md §13 for the measured aggregate rates against sweeping the chains one after
     another, with built-in and with user types (cfg2 with two user types: 1.6x at C = 2, 3.7x at C = 8 over sequential
-    spec; a one-chain group measured 0.997x, and ``chains=1`` runs no group)."""
+    spec; a one-chain group measured 0.997x, and ``chains=1`` runs no group).
+
+    ``summary=S`` (a ``capi.PosteriorSummary`` with K datasets, n_obs observations, at least C chains and labels up to
+    at least N): chain c also offers every row it writes to its CSV file, the initial row included, to S as chain c, so
+    that PSMs, the least-squares consensus and the chains' agreement are at hand without reading the files back (S
+    applies its own burnin / thin to the rows offered).  Not with ``distributed``."""
     if reference_literal:  # the literal reference in one switch: never-refreshed gamma table, trajectories not permuted
         stale_gamma_table, sstar_compat, factorised = True, True, False
     t_entry = time.perf_counter()
@@ -613,6 +710,13 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
         fsel = list(featureSelect) if featureSelect is not None else [None] * C
         if len(outputs) != C or len(fsel) != C:
             raise ValueError(f"chains={C}: outputFile (and featureSelect when given) need {C} paths")
+    if summary is not None:
+        if distributed:
+            raise ValueError("summary= takes the allocations of one GPU's chains; with distributed=True read the CSV "
+                             "file back (generate_psm)")
+        if (summary.K, summary.n) != (K, n_obs) or summary.chains < C or summary.N < N:
+            raise ValueError(f"summary has K={summary.K}, n_obs={summary.n}, {summary.chains} chains, N={summary.N}; "
+                             f"this run needs K={K}, n_obs={n_obs}, >= {C} chains, N >= {N}")
     # the N^K-row tables of :69-92 where they are small, the factorised sums (FactorisedZ) otherwise
     if factorised is None:
         factorised = N ** K > 200_000
@@ -642,9 +746,12 @@ def pmdi(dataFiles, dataTypes, N, particles, rho, iter, outputFile, *, thin=1, f
         if C > 1:
             group = capi.Group([ch.ctx for ch in chain_list])
         t0 = time.perf_counter()
-        for ch in chain_list:
+        for c, ch in enumerate(chain_list):
             ch.stats["setup_s"] = t0 - t_entry  # data to the device, pool allocation (and a user type's compilation)
             ch.out.write(csv_row(ch.M, ch.phi, 0, ch.s) + "\n")  # :158
+            if summary is not None:
+                ch.offer = (lambda a, c=c: summary.add(c, a))
+                ch.offer(ch.s)
         for it in range(1, iter + 1):                             # :164
             args = [ch.sweep_args(it) for ch in chain_list]
             if group is not None:
