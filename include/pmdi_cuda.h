@@ -86,6 +86,18 @@ int pmdi_ipc_import(pmdi_ctx* ctx, const void* handles /* n_ranks x PMDI_IPC_HAN
 #define PMDI_ENGINE_SPEC 2
 int pmdi_ctx_set_engine(pmdi_ctx* ctx, int32_t engine);
 
+/*
+ * Whether the context sweeps with the wide kernels (*wide = 1) or the staged ones (0); valid once the context is
+ * prepared (its first upload, sweep, feature, cluster-eval or IPC export call).  The pool and spec sweeps stage each
+ * observation over all datasets in shared memory, two deep, beside their tables.  A context is wide when that does
+ * not fit with its N and particle count, or when a dataset has more than 8,192 features; its sweeps then read the
+ * observation from global memory instead, with the same results.  The choice is automatic.  PMDI_ENGINE=dense on a
+ * wide context runs the pool engine (pmdi_sweep_out.engine says so).  Wide contexts are not yet supported in groups
+ * (pmdi_group_create refuses such a member, naming it) or with their particles sharded over GPUs (refused when the
+ * context is prepared).
+ */
+int pmdi_ctx_is_wide(const pmdi_ctx* ctx, int32_t* wide);
+
 /* Use an externally owned cudaStream_t (e.g. the host framework's current stream). */
 int pmdi_ctx_set_stream(pmdi_ctx* ctx, void* cuda_stream);
 void* pmdi_ctx_get_stream(pmdi_ctx* ctx);
@@ -95,7 +107,9 @@ void* pmdi_ctx_get_stream(pmdi_ctx* ctx);
  * `data` is a HOST column-major n_obs x D matrix with leading dimension `ld` (Julia
  * Matrix{Float64} for PMDI_GAUSSIAN, Matrix{Int64} for the others: levels 1..L for
  * categorical, counts >= 0 for negative-binomial).  It is copied to the device; the caller
- * keeps ownership.  All feature flags are reset to true.
+ * keeps ownership.  All feature flags are reset to true.  1 <= D <= 65,536 features per dataset; the total width
+ * over the datasets is limited by device memory alone (the context's arena grows linearly with every D: the
+ * preparing call fails with the bytes it needs and the bytes free when they do not fit).
  */
 int pmdi_set_dataset(pmdi_ctx* ctx, int32_t k, int32_t type_tag, int32_t elem_kind,
                      const void* data, int64_t n_obs, int64_t D, int64_t ld);
@@ -203,8 +217,8 @@ int pmdi_sweep_download(pmdi_ctx* ctx, pmdi_sweep_out* out);         /* sync + d
  *                      the grid it has alone when the grids fit side by side, otherwise a share of the SM count in
  *                      proportion to those grids (two 117-CTA members: 74 CTAs each).  Its role split and shared
  *                      memory follow the share; a member whose share is too small for it (at least one proposal, one
- *                      evaluation and the deciding CTA, and its tables in shared memory) makes the create fail with a
- *                      message that names it, and nothing changes.
+ *                      evaluation and the deciding CTA, and its tables in shared memory), or that would be wide at its
+ *                      share (pmdi_ctx_is_wide), makes the create fail with a message that names it, and nothing changes.
  *   pmdi_group_run     after pmdi_sweep_upload on every member: each member's set-up kernels, one launch of the
  *                      group kernel, each member's finish, all on the group's own stream (it waits for the members'
  *                      uploads); then pmdi_sweep_download on each member as after pmdi_sweep_run.  A member's

@@ -5,6 +5,8 @@
 #pragma once
 #include "pool_types.cuh"
 
+#ifndef PMDI_X_GLOBAL  // (the wide module, sweep_wide.cu, carries only k_eval_row_wide from here: at the end)
+
 // all rows of a dataset to the empty-cluster state (constructors gaussian_cluster.jl:17-21,
 // categorical_cluster.jl:6-10, negbinom_cluster.jl:9-10)
 extern "C" __global__ void k_init_rows(DsDev ds, long long rows) {
@@ -501,3 +503,42 @@ extern "C" __global__ void k_cluster_n(SweepParams sp, long long* cluster_n) {
     cluster_n[idx] = v;
   }
 }
+#else
+
+// k_eval_row for a dataset whose row does not fit in shared memory: the same operators, with the observation read
+// from global memory (DsDev::xstage: the flags of Categorical / NegBinom data are folded in, as k_eval_row folds
+// them while it stages).  One warp.
+extern "C" __global__ void k_eval_row_wide(SweepParams sp, int k, int obs, double* out) {
+  const DsDev& ds = sp.ds[k];
+  const int lane = threadIdx.x;
+  const unsigned char* xs = (const unsigned char*)ds.xstage + (size_t)obs * ds.Dp * PMDI_XBYTES(ds);
+  const long long row = sp.proto_base;
+  const int n = ds.n[row];
+  double acc = ds.rc[n];
+  for (int j = 0; j < ds.J; ++j) {
+    double v;
+#ifdef PMDI_USER_TYPES
+    if (ds.type == T_USER) {
+      const int fo = j * ds.FB + 2 * lane;
+      const int nits = min(ds.FB / PMDI_WF, (ds.Dp - j * ds.FB) / PMDI_WF);
+      double unused;
+      v = user_block(ds, ds.ust + row * user_row_words(ds) + fo, 0, ds.flag + fo, nits, 0, n, xs,
+                     xs + fo * (ds.uW < 0 ? 4u : 8u), &unused);
+    } else
+#endif
+    if (ds.type == T_GAUSSIAN) v = gauss_eval_block(ds, row, j, n, (const double*)xs, lane);
+    else if (ds.type == T_CATEGORICAL && sp.engine) {
+      const PoolDev& pd = sp.pd[k];
+      const int base = j * ds.FB + 2 * lane;
+      const int nits = min(ds.FB / PMDI_WF, (ds.Dp - j * ds.FB) / PMDI_WF);
+      double unused;
+      v = cat_block(pd.cw + ((size_t)row * ds.Dp + base) * pd.wpf, 0, pd.wpf, pd.fpw, nits, 0, xs, xs + base * 4u,
+                    &unused);
+    }
+    else if (ds.type == T_CATEGORICAL) v = cat_eval_block(ds, row, j, (const int*)xs, lane);
+    else v = nb_eval_block(ds, row, j, n, (const int*)xs, lane, sp.lf_glob, sp.lf_glob_T);
+    acc += v;
+  }
+  if (lane == 0) *out = acc;
+}
+#endif

@@ -336,6 +336,21 @@ __device__ __forceinline__ double lds_f64(unsigned a) {
   return v;
 }
 
+// How the pool and spec block operators (pool_types.cuh, user_type.cuh) address the observation.  By default it is
+// staged in shared memory: PMDI_XADDR is a 32-bit shared address and the loads are ld.shared.  With PMDI_X_GLOBAL
+// (the wide kernels, sweep_wide.cu: an observation too wide to stage) PMDI_XADDR is a byte pointer into
+// DsDev::xstage and the loads are read-only global loads.  Without the macro the names expand to exactly the tokens
+// the operators had before, so the staged kernels keep their code.
+#ifdef PMDI_X_GLOBAL
+#define PMDI_XADDR const unsigned char*
+#define PMDI_LDX_F64X2(a_) __ldg((const double2*)(a_))
+#define PMDI_LDX_I32X2(a_) __ldg((const int2*)(a_))
+#else
+#define PMDI_XADDR unsigned
+#define PMDI_LDX_F64X2(a_) lds_f64x2(a_)
+#define PMDI_LDX_I32X2(a_) lds_i32x2(a_)
+#endif
+
 // mu / lm / flag / xs point at this lane's first feature of the item; nits 64-feature iterations.
 __device__ __noinline__ double gauss_eval_raw(const double* mu, const double* lm, const double* aux,
                                               const uint8_t* flag /* NULL: all on */, unsigned xs, int nits,

@@ -44,6 +44,11 @@
 #define POOL_BIG_REF (1 << 30)
 #define POOL_FLAG_SHIFT 44  // grid counter: arrivals in the low 44 bits, resampling decisions above
 #define POOL_ARRIVE_MASK ((1ull << POOL_FLAG_SHIFT) - 1ull)
+#ifdef PMDI_X_GLOBAL
+#define POOL_RB 256  // blocks of a row whose partials meet in shared memory: 65,536 features in 256-feature blocks
+#else
+#define POOL_RB 32   // ... 8,192 features (a wider dataset runs the wide kernels)
+#endif
 
 struct PoolSmem {
   unsigned long long obs_bar[PMDI_OBS_RING];
@@ -51,7 +56,7 @@ struct PoolSmem {
   unsigned long long xepoch;   // cross-rank barrier arrivals expected so far (one per rank)
   unsigned long long flag_base;  // resampling decisions attached to the counter before this sweep
   double res_mx;
-  double red[2][2][32];        // [row-iteration parity][updated or plain / split source][block] partials
+  double red[2][2][POOL_RB];   // [row-iteration parity][updated or plain / split source][block] partials
   int res_flag;                // the last resolved step resamples
   int res_next;                // CTA 0: the decision to attach to the next B1 arrival
   int fail;
@@ -145,8 +150,12 @@ __device__ __noinline__ void pool_eval_rows(const SweepParams& sp, PoolSmem& sm,
   const int jq = sp.jq, rpc = PMDI_NW / jq;
   const int sub = warp / jq, wj = warp - sub * jq;
   const int total = sm.rbase[b][K];
+#ifdef PMDI_X_GLOBAL  // x[st] and x[st-1] are read from global memory: their observations
+  const int oc = sp.order[sp.n1 - 1 + st], op = st > 0 ? sp.order[sp.n1 - 2 + st] : oc;
+#else
   const unsigned xc = (unsigned)__cvta_generic_to_shared(xring + (size_t)(st % sp.obs_ring) * sp.sm_x_bytes);
   const unsigned xp = (unsigned)__cvta_generic_to_shared(xring + (size_t)((st + sp.obs_ring - 1) % sp.obs_ring) * sp.sm_x_bytes);
+#endif
   int buf = 0;
 #pragma unroll 1
   for (int base = (int)blockIdx.x * rpc; base < total; base += sp.G * rpc, buf ^= 1) {
@@ -159,6 +168,7 @@ __device__ __noinline__ void pool_eval_rows(const SweepParams& sp, PoolSmem& sm,
       const DsDev& ds = sp.ds[k];
       const PoolDev& pd = sp.pd[k];
       if (wj < ds.J) {
+#ifndef PMDI_X_GLOBAL
         if (obs_ok < st) {  // x[st] has landed in the ring (x[st-1] was waited for one step ago)
           if (lane == 0) {
 #pragma unroll 1
@@ -169,6 +179,7 @@ __device__ __noinline__ void pool_eval_rows(const SweepParams& sp, PoolSmem& sm,
           __syncwarp();
           obs_ok = st;
         }
+#endif
         c = ldcg_i32(pd.live + (idx - sm.rbase[b][k]));
         int tot = 0;  // the row's bookkeeping words in one round trip
         nc = ldcg_i32(ds.n + c);
@@ -178,7 +189,14 @@ __device__ __noinline__ void pool_eval_rows(const SweepParams& sp, PoolSmem& sm,
         // every reference chose it: in place (src/pmdi.jl:284-286); some did: split (:288-309)
         mode = tot == 0 ? 0 : (tot == rf ? 1 : 2);
         if (mode != 2) d = c;
+#ifdef PMDI_X_GLOBAL
+        const size_t xrow = (size_t)ds.Dp * PMDI_XBYTES(ds);  // this dataset's rows are an array of their own
+        const unsigned char* const xc = (const unsigned char*)ds.xstage + (size_t)oc * xrow;
+        const unsigned char* const xp = (const unsigned char*)ds.xstage + (size_t)op * xrow;
+        const unsigned xo = 0u;
+#else
         const unsigned xo = (unsigned)ds.x_off;
+#endif
 #pragma unroll 1
         for (int j = wj; j < ds.J; j += jq) {
           const int q0 = j * ds.FB;
@@ -716,7 +734,11 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
   // dynamic shared memory: [observation ring][lf table][lp scratch][Pi][lw][inc][unit tables]
   unsigned char* xring = smem_raw;
   PoolTables T;
+#ifdef PMDI_X_GLOBAL
+  T.lf = (double*)smem_raw;  // (no observation ring)
+#else
   T.lf = (double*)(smem_raw + (size_t)sp.obs_ring * sp.sm_x_bytes);
+#endif
   T.lp_s = T.lf + sp.lf_T;
   T.Pi_s = T.lp_s + (size_t)NW * Npad;
   T.lw_s = T.Pi_s + (size_t)K * N;
@@ -748,15 +770,19 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
     sm.res_flag = 0; sm.res_next = 0; sm.fail = 0; sm.ev = 0; sm.pdone = 0; sm.res_mx = 0.0;
     const unsigned long long b0 = __ldcg(sp.bar_state);  // the counters run on from the previous sweep
     sm.epoch = b0 & POOL_ARRIVE_MASK; sm.flag_base = b0 >> POOL_FLAG_SHIFT; sm.xepoch = __ldcg(sp.bar_state + 1);
+#ifndef PMDI_X_GLOBAL
 #pragma unroll 1
     for (int b = 0; b < sp.obs_ring; ++b) mbar_init(&sm.obs_bar[b], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+#endif
   }
   if (warp == NW - 1) pool_snapshot(sp, sm, 0);
   __syncthreads();
+#ifndef PMDI_X_GLOBAL
   if (tid == 0)
 #pragma unroll 1
     for (int s = 0; s < sp.obs_ring; ++s) pool_issue_obs(sp, s, xring, sm.obs_bar);
+#endif
   pool_load_units(sp, sm, T, ns);
 
   const bool timing = DBG && sp.phase_ns != nullptr;
@@ -779,7 +805,9 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
     SWEEP_TRACE(t, 40)
     // ---- P(t): the last warp keeps house, the others propose
     if (t > 0) {
+#ifndef PMDI_X_GLOBAL
       if (tid == PMDI_NT - 1) pool_issue_obs(sp, t - 1 + sp.obs_ring, xring, sm.obs_bar);  // x[t-1] is dead: its slot refills
+#endif
       pool_duties(sp, T, nu, par ^ 1);
       if (sp.R > 1) {  // the ranks' partials of step t-1 have had E(t) to arrive
         if (warp == NW - 1) pool_resolve_ranks(sp, sm, t - 1);
@@ -867,6 +895,16 @@ __device__ __forceinline__ void pool_sweep_body(const SweepParams& sp, PoolSmem&
   }                                                                                                       \
   __syncthreads();
 
+#ifdef PMDI_X_GLOBAL  // (the wide module, sweep_wide.cu: the observation is read from global memory)
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool_wide(const __grid_constant__ SweepParams sp_in) {
+  POOL_KERNEL_PROLOGUE
+  pool_sweep_body<false>(sp_s, sm, smem_raw, s_tmp);
+}
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool_wide_dbg(const __grid_constant__ SweepParams sp_in) {
+  POOL_KERNEL_PROLOGUE
+  pool_sweep_body<true>(sp_s, sm, smem_raw, s_tmp);
+}
+#else
 // production kernel: no debug capture, no tracing, no phase timing in the instruction stream
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_pool(const __grid_constant__ SweepParams sp_in) {
   POOL_KERNEL_PROLOGUE
@@ -918,3 +956,4 @@ extern "C" __global__ void k_pool_init(SweepParams sp) {
   __syncthreads();
   if (t == 0) { pd.refcnt[pd.cap - 1] = POOL_BIG_REF; ds.n[pd.cap - 1] = 0; }
 }
+#endif

@@ -38,7 +38,7 @@
 __device__ __noinline__ double gauss_block(const double* s_sum, const double* s_beta, const double* s_mu,
                                            const double* s_lamn, long long d_off /* dst - src, elements */,
                                            const double* s_aux, double* d_aux, const uint8_t* flag_p, int nit,
-                                           int mode, int n, unsigned xp, unsigned xc, double* v_src) {
+                                           int mode, int n, PMDI_XADDR xp, PMDI_XADDR xc, double* v_src) {
   const double nn = (double)(n + 1);  // size after the add
   double c1 = 0, c2 = 0, c3 = 0, c4 = 0, c5 = 0, c6 = 0, r2 = 0, r3 = 0, r6 = 0;
   if (mode) {
@@ -65,9 +65,9 @@ __device__ __noinline__ double gauss_block(const double* s_sum, const double* s_
     for (int i = 0; i < 2; ++i)
       if (h + i < nit) {
         const int o = (h + i) * PMDI_WF;
-        const double2 y = lds_f64x2(xc + o * 8);
+        const double2 y = PMDI_LDX_F64X2(xc + o * 8);
         double2 x = make_double2(0.0, 0.0);
-        if (mode) x = lds_f64x2(xp + o * 8);
+        if (mode) x = PMDI_LDX_F64X2(xp + o * 8);
         const uchar2 fl = *(const uchar2*)(flag_p + o);
         PMDI_GAUSS_FEATURE(x)
         PMDI_GAUSS_FEATURE(y)
@@ -98,24 +98,24 @@ __device__ __noinline__ double gauss_block(const double* s_sum, const double* s_
 #undef PMDI_GAUSS_FEATURE
 
 // ------------------------------------------------------------------------------------------
-// NegBinom.  S pointers at this lane's first feature; observations by shared-memory address; n =
+// NegBinom.  S pointers at this lane's first feature; observations by PMDI_XADDR (cluster_types.cuh); n =
 // size of the source row.  Partials include the row's aux (the x-independent part).
 // ------------------------------------------------------------------------------------------
 __device__ __noinline__ double nb_block(const long long* s_S, long long d_off, const double* s_aux, double* d_aux,
-                                        int nit, int mode, int n, unsigned xp, unsigned xc, unsigned lf_s, int T,
+                                        int nit, int mode, int n, PMDI_XADDR xp, PMDI_XADDR xc, unsigned lf_s, int T,
                                         double* v_src) {
   double aux = 0.0, ed = 0.0, es = 0.0;
   const long long ns2 = n + 2, nd2 = n + 3, na = n + 2;  // source: n+2; after the add: size n+1
 #pragma unroll 1
   for (int it = 0; it < nit; ++it) {
     longlong2 s = ldcg_i64x2(s_S + it * PMDI_WF);
-    const int2 y = lds_i32x2(xc + it * PMDI_WF * 4);
+    const int2 y = PMDI_LDX_I32X2(xc + it * PMDI_WF * 4);
     if (mode != 1) {
       if (y.x >= 0) { const long long b = s.x + y.x; es += lfact_s(b, lf_s, T) - lfact_s(b + ns2, lf_s, T); }
       if (y.y >= 0) { const long long b = s.y + y.y; es += lfact_s(b, lf_s, T) - lfact_s(b + ns2, lf_s, T); }
     }
     if (mode) {
-      const int2 x = lds_i32x2(xp + it * PMDI_WF * 4);
+      const int2 x = PMDI_LDX_I32X2(xp + it * PMDI_WF * 4);
       if (x.x >= 0) { s.x += x.x; aux += lfact_s(s.x + na, lf_s, T) - lfact_s(s.x, lf_s, T); }
       if (x.y >= 0) { s.y += x.y; aux += lfact_s(s.y + na, lf_s, T) - lfact_s(s.y, lf_s, T); }
       *(longlong2*)(const_cast<long long*>(s_S) + d_off + it * PMDI_WF) = s;
@@ -154,14 +154,14 @@ __device__ __forceinline__ double cat_field(unsigned long long w, int f, int fpw
 }
 
 __device__ __noinline__ double cat_block(const unsigned long long* s_cw, long long d_off /* words */, int wpf, int fpw,
-                                         int nit, int mode, unsigned xp, unsigned xc, double* v_src) {
+                                         int nit, int mode, PMDI_XADDR xp, PMDI_XADDR xc, double* v_src) {
   const int fw = 64 / fpw;
   double pd = 1.0, ps = 1.0;
 #pragma unroll 1
   for (int it = 0; it < nit; ++it) {
-    const int2 y = lds_i32x2(xc + it * PMDI_WF * 4);
+    const int2 y = PMDI_LDX_I32X2(xc + it * PMDI_WF * 4);
     int2 x = make_int2(0, 0);
-    if (mode) x = lds_i32x2(xp + it * PMDI_WF * 4);
+    if (mode) x = PMDI_LDX_I32X2(xp + it * PMDI_WF * 4);
     if (wpf == 1) {
       ulonglong2 w = ldcg_u64x2(s_cw + (size_t)it * PMDI_WF);
       if (mode != 1) {

@@ -45,12 +45,17 @@
 
 #define SPEC_FC 256      // free-row ids per dataset cached by an E-CTA (shared memory)
 #define SPEC_EC 512      // entries of the live-row list kept in shared memory (the rest spills to HBM)
+#ifdef PMDI_X_GLOBAL
+#define SPEC_RB 512      // blocks of a row whose partials meet in shared memory: 65,536 features in 128-feature blocks
+#else
+#define SPEC_RB 64       // ... 8,192 features (a wider dataset runs the wide kernels)
+#endif
 
 struct SpecSmem {
   unsigned long long obs_bar[PMDI_OBS_RING];
   unsigned long long epoch, xepoch;
   double res_mx;
-  double red[2][2][64];
+  double red[2][2][SPEC_RB];
   int res_flag;
   int fail;
   int ev;
@@ -640,8 +645,12 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
   const int jq = sp.jq, rpc = PMDI_NW / jq;
   const int sub = warp / jq, wj = warp - sub * jq;
   const int n_list = sm.cnt, total = n_list + K, lp = sm.lpar;
+#ifdef PMDI_X_GLOBAL  // x[st] and x[st-1] are read from global memory: their observations
+  const int oc = sp.order[sp.n1 - 1 + st], op = st > 0 ? sp.order[sp.n1 - 2 + st] : oc;
+#else
   const unsigned xc = (unsigned)__cvta_generic_to_shared(xring + (size_t)(st % sp.obs_ring) * sp.sm_x_bytes);
   const unsigned xp = (unsigned)__cvta_generic_to_shared(xring + (size_t)((st + sp.obs_ring - 1) % sp.obs_ring) * sp.sm_x_bytes);
+#endif
   const int mode = st == 0 ? 0 : 2;
   int buf = 0;
 #pragma unroll 1
@@ -662,6 +671,12 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
       SCHECK(k >= 0 && k < K && v >= 0 && v < pd.cap && (mode == 0 || (c >= 0 && c < pd.cap - 1 && c != v)) && nc >= 0 && nc <= sp.n_obs, 91)
       if (sm.fail) { active = false; }
       if (active && wj < ds.J) {
+#ifdef PMDI_X_GLOBAL
+        const size_t xrow = (size_t)ds.Dp * PMDI_XBYTES(ds);  // this dataset's rows are an array of their own
+        const unsigned char* const xc = (const unsigned char*)ds.xstage + (size_t)oc * xrow;
+        const unsigned char* const xp = (const unsigned char*)ds.xstage + (size_t)op * xrow;
+        const unsigned xo = 0u;
+#else
         if (obs_ok < st) {  // x[st] has landed in the ring (x[st-1] was waited for one step ago)
           if (lane == 0) {
 #pragma unroll 1
@@ -672,6 +687,7 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
           obs_ok = st;
         }
         const unsigned xo = (unsigned)ds.x_off;
+#endif
         if (wj == 0 && lane < 2) rcv = __ldg(ds.rc + nc + 1 - lane);  // lane 1: the row's size constant, lane 0: its child's
         SWEEP_TRACE(st - 1, 63)
 #pragma unroll 1
@@ -1045,7 +1061,11 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   // dynamic shared memory: [observation ring][lf table][role tables]
   unsigned char* xring = smem_raw;
   SpecTables T;
+#ifdef PMDI_X_GLOBAL
+  T.lf = (double*)smem_raw;  // (no observation ring)
+#else
   T.lf = (double*)(smem_raw + (size_t)sp.obs_ring * sp.sm_x_bytes);
+#endif
   unsigned char* rt = (unsigned char*)(T.lf + ((sp.lf_T + 1) & ~1));  // 16-byte aligned
   T.lp_s = (double*)rt;
   T.Pi_s = T.lp_s + (size_t)NW * Npad;
@@ -1073,8 +1093,10 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
     sm.res_flag = 0; sm.fail = 0; sm.ev = 0; sm.pdone = 0; sm.res_mx = 0.0;
     sm.epoch = __ldcg(sp.bar_state); sm.xepoch = __ldcg(sp.bar_state + 1);  // the counters run on from the previous sweep
     sm.lpar = 0; sm.cnt = 0;
+#ifndef PMDI_X_GLOBAL
     for (int b = 0; b < sp.obs_ring; ++b) mbar_init(&sm.obs_bar[b], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+#endif
   }
   __syncthreads();
   if (is_p) {
@@ -1086,8 +1108,10 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
     for (int u = tid; u < nu; u += PMDI_NT) T.u_ks[u] = (u % K) | ((u / K) << 8);
     spec_load_units<GRP>(sp, sm, T, ns);
   } else if (cta != sp.G - 1) {
+#ifndef PMDI_X_GLOBAL
     if (tid == 0)
       for (int s = 0; s < sp.obs_ring; ++s) pool_issue_obs(sp, s, xring, sm.obs_bar);
+#endif
 #pragma unroll 1
     for (int i = tid; i < sp.lf_T; i += PMDI_NT) T.lf[i] = sp.lf_glob[i];
     const int nl = ldcg_i32(sp.gcnt);  // the set-up kernel listed the live prefix rows
@@ -1160,7 +1184,9 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
       }
     } else {
       // ---- E side: outcome of step t-1, then the children of step t and the predictive of x[t+1]
+#ifndef PMDI_X_GLOBAL
       if (tid == PMDI_NT - 1 && t > 0) pool_issue_obs(sp, t - 1 + sp.obs_ring, xring, sm.obs_bar);  // x[t-1]'s slot refills
+#endif
       if (t > 0) spec_fix<DBG>(sp, sm, T, e, t - 1);
       else spec_refresh_children(sp, sm, T, e);
       // the distinct clusters the reference evaluates at step t (src/pmdi.jl:218-220): the list and the empty one
@@ -1220,7 +1246,16 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   }                                                                                                       \
   __syncthreads();
 
-#ifndef PMDI_SPEC_GROUP  // (the group module, spec_group.cu, carries the group kernels alone)
+#if defined(PMDI_X_GLOBAL)  // (the wide module, sweep_wide.cu: the observation is read from global memory)
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_wide(const __grid_constant__ SweepParams sp_in) {
+  SPEC_KERNEL_PROLOGUE
+  spec_sweep_body<false, false>(sp_s, sm, smem_raw, s_tmp);
+}
+extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec_wide_dbg(const __grid_constant__ SweepParams sp_in) {
+  SPEC_KERNEL_PROLOGUE
+  spec_sweep_body<true, false>(sp_s, sm, smem_raw, s_tmp);
+}
+#elif !defined(PMDI_SPEC_GROUP)  // (the group module, spec_group.cu, carries the group kernels alone)
 extern "C" __global__ void __launch_bounds__(PMDI_NT, 1) k_sweep_spec(const __grid_constant__ SweepParams sp_in) {
   SPEC_KERNEL_PROLOGUE
   spec_sweep_body<false, false>(sp_s, sm, smem_raw, s_tmp);

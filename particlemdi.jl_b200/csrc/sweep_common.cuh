@@ -36,6 +36,7 @@ __device__ __forceinline__ bool mbar_try_wait(unsigned long long* bar, unsigned 
   return ok != 0;
 }
 
+#ifndef PMDI_X_GLOBAL  // (the wide kernels read the observation from global memory: no ring)
 // pool and spec: one thread bulk-copies the K rows of the observation swept at `step` into its ring slot
 __device__ __noinline__ void pool_issue_obs(const SweepParams& sp, int step, unsigned char* xring,
                                             unsigned long long* bars) {
@@ -58,6 +59,7 @@ __device__ __noinline__ void pool_issue_obs(const SweepParams& sp, int step, uns
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
   }
 }
+#endif
 
 // pool and spec: optional per-warp event trace of one CTA and one step (PMDI_TRACE_STEP): tag << 48 | clock64; stores
 // only.  Smem: the engine's shared-memory struct (tr_n[PMDI_NW]: events per warp).

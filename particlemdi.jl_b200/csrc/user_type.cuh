@@ -31,18 +31,24 @@
 PMDI_USER_TYPE_LIST(PMDI_USER_CHECK)
 #undef PMDI_USER_CHECK
 
-__device__ __forceinline__ double user_x(const DsDev& ds, unsigned xs_addr, int f, int x_is_int) {
+__device__ __forceinline__ double user_x(const DsDev& ds, PMDI_XADDR xs_addr, int f, int x_is_int) {
   // staged observation: doubles, or 32-bit integers for integer-valued data
+#ifdef PMDI_X_GLOBAL
+  if (x_is_int) return (double)__ldg((const int*)(xs_addr + f * 4u));
+  return __ldg((const double*)(xs_addr + f * 8u));
+#else
   if (x_is_int) { int v; asm("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(xs_addr + f * 4u)); return (double)v; }
   double v; asm("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(xs_addr + f * 8u)); return v;
+#endif
 }
 
 // One block of one row, by one warp: mode 0 plain evaluation, 1 add + evaluation, 2 add into the row
 // d_off doubles further on + evaluation of both (pool_types.cuh).  s_st at the row's word 0, this lane's
-// first feature; xp / xc: shared-memory addresses of the block's first feature of this lane.
+// first feature; xp / xc: addresses of the block's first feature of this lane in the staged observation (PMDI_XADDR:
+// shared memory, or global memory in the wide kernels).
 template <class U>
 __device__ __forceinline__ double user_block_t(const DsDev& ds, const double* s_st, long long d_off, const uint8_t* flag_p,
-                                               int nit, int mode, int n, unsigned xp, unsigned xc, double* v_src) {
+                                               int nit, int mode, int n, PMDI_XADDR xp, PMDI_XADDR xc, double* v_src) {
   const int W = U::WORDS, Dp = ds.Dp, xi = ds.uW < 0;
   double ed = 0.0, es = 0.0;
 #pragma unroll 1
@@ -80,7 +86,7 @@ __device__ __forceinline__ double user_block_t(const DsDev& ds, const double* s_
 // the block operator of the dataset's type; d_off / the row offset of s_st are in units of the type's row
 // (WORDS * Dp doubles), which the caller computes from |ds.uW|
 __device__ __noinline__ double user_block(const DsDev& ds, const double* s_st, long long d_off, const uint8_t* flag_p,
-                                          int nit, int mode, int n, unsigned xp, unsigned xc, double* v_src) {
+                                          int nit, int mode, int n, PMDI_XADDR xp, PMDI_XADDR xc, double* v_src) {
   switch (PMDI_USER_SLOT(ds)) {
 #define PMDI_USER_CASE(s_, U_) \
     case s_: return user_block_t<U_>(ds, s_st, d_off, flag_p, nit, mode, n, xp, xc, v_src);
