@@ -840,10 +840,16 @@ __device__ __noinline__ void spec_row_pull(const SweepParams& sp, int4 j0, int4 
 // or next child) go back to the free lists; the list of live rows is rebuilt.  The children of step
 // st+1 were computed before the call and stay valid: a row's content does not depend on who refers
 // to it.
+// With the particles sharded over several GPUs (sp.R > 1) this is the whole-pool form below: rows of
+// another rank's ancestors are pulled, and every rank recounts, marks and rescans its whole pool.  On
+// one GPU spec_resample (after it) does the same in proportion to the live rows.
+// Only spec_resample calls this, and only with sp.R > 1: the `sp.R > 1` test below and spec_xsync's
+// one-GPU branch are always taken / never taken here.  They are left as they were so that the sharded
+// event runs the code it ran when it also served one GPU (no multi-GPU machine checked a rewrite).
 // ------------------------------------------------------------------------------------------------
 template <bool GRP>
-__device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int ns, int st,
-                                           int* s_tmp, bool is_p, int e) {
+__device__ __forceinline__ bool spec_resample_sharded(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int ns,
+                                                   int st, int* s_tmp, bool is_p, int e) {
   const int K = sp.K, N = sp.N, Ps = sp.Ps;
   const int ev = sm.ev;
   const long long gt = (long long)spec_cta<GRP>() * PMDI_NT + threadIdx.x, GT = (long long)sp.G * PMDI_NT;
@@ -1045,6 +1051,201 @@ __device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, 
   return !sm.fail;
 }
 
+// The resampling on one GPU.  What may be live afterwards is known without looking at the pool: the particles' new
+// row maps are copies of old ones, and an old row map refers only to rows of the live-row list (after the fix of
+// step st, the copy every E-CTA holds, in the same order) or to the empty row.  Every other row id of a dataset is
+//   - on the free stack or in an E-CTA's free-id cache,
+//   - the child of step st+1 of a listed row (the entry's .y, computed by E'(st+2)) or one of the two ids E'(st+2)
+//     handed out for step st+2 (info[st&1].child of the row and of that child), or
+//   - the empty row or an id handed out for it (its children stay reserved whatever the resampling does).
+// So only the listed rows need a recount, and a listed row nobody refers to any more frees exactly itself, its child
+// and their two ids of step st+2 (none were handed out when st+2 is past the last step).  The caches and the free
+// stack are left as they are: the ids in them were free before and stay free.  The choice counters that can be
+// non-zero are those the particles raised at steps st and st+1 (each unit's u_c2, u_c1: a commit clears its unit's
+// counter of two steps ago): the units clear them themselves.  The empty row's reference count is read by nobody
+// (a birth is decided from its choice counter) and is not counted.
+// Three grid barriers: the plan (its inputs are complete since the decision) is drawn before the first one; row
+// maps and the reset of the listed rows' counts; the recount; then each E-CTA drops the dead rows from its copy of
+// the list, and the CTA that owns a dead entry (index mod GE) frees its four ids into its cache.  At the final
+// resampling (st+1 == steps) only the row maps are needed: the next sweep's set-up starts the pool afresh.
+template <bool GRP>
+__device__ __noinline__ bool spec_resample(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int ns, int st,
+                                           int* s_tmp, bool is_p, int e) {
+  if (sp.R > 1) return spec_resample_sharded<GRP>(sp, sm, T, ns, st, s_tmp, is_p, e);
+  const int K = sp.K, N = sp.N, P = sp.P, GE = sp.G - sp.GP - 1;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int ev = sm.ev;
+  const long long gt = (long long)spec_cta<GRP>() * PMDI_NT + tid, GT = (long long)sp.G * PMDI_NT;
+  const int parn = (st + 1) & 1;  // the copy of the reference counts the fix of step st+1 reads
+  const bool has_next = st + 1 < sp.steps;
+  // sub-phase timers (instrumented runs): tacc[4] plan + first barrier, [5] row maps + recount, [7] list rebuild
+  const bool tm = sp.phase_ns != nullptr && tid == 0;
+  unsigned long long t_ = tm ? globaltimer_ns() : 0ull;
+#define RS_MARK(i_) if (tm) { const unsigned long long n_ = globaltimer_ns(); sm.tacc[i_] += (n_ - t_) * PMDI_NW; t_ = n_; }
+  if (spec_cta<GRP>() == sp.G - 1) {  // the D-CTA: its dynamic shared memory is free for the plan
+    extern __shared__ __align__(16) unsigned char plan_raw[];
+    PlanScratch sc = {sp.sc_w, sp.sc_pp, sp.sc_u, sp.sc_j, sp.sc_anc0};
+    if (sp.plan_smem) {
+      sc.w = (double*)plan_raw; sc.pp = sc.w + P; sc.u = sc.pp + P;
+      sc.j = (int*)(sc.u + P); sc.a0 = sc.j + P;
+    }
+    pool_resample_plan(sp, st, ev, sm.res_mx, s_tmp, sp.lw + (size_t)(st & 1) * P, sc);
+  }
+  // every E-CTA has finished E'(st+2) and the fix of step st, every commit of step st+1 is in, the plan is drawn
+  if (!spec_gsync(sp, sm)) return false;
+  RS_MARK(4)
+  const int* anc = sp.anc_log + (size_t)ev * P;
+#pragma unroll 1
+  for (int k = 0; k < K; ++k) {
+    const PoolDev& pd = sp.pd[k];
+    const int* rm_old = pd.rowmap + (size_t)(ev & 1) * P * N;
+    int* rm_new = pd.rowmap + (size_t)((ev + 1) & 1) * P * N;
+#pragma unroll 1
+    for (long long i = gt; i < (long long)P * N; i += GT) {
+      const int p = (int)(i / N), m = (int)(i - (long long)p * N);
+      __stcg(rm_new + i, ldcg_i32(rm_old + (size_t)(ldcg_i32(anc + p) - 1) * N + m));
+    }
+  }
+  if (is_p)
+    for (int sl = tid; sl < ns; sl += PMDI_NT) T.lw_s[sl] = 1.0;  // logweight .= 1.0 (src/pmdi.jl:319)
+  if (tid == 0) { sm.ev = ev + 1; sm.res_flag = 0; }  // (read after the next CTA barrier: the new row maps)
+  if (!has_next) {  // the final resampling: the row maps are all the finish kernel reads
+    __syncthreads();
+    return !sm.fail;
+  }
+  const int b3 = st % 3, z3 = (st + 1) % 3;
+  if (is_p) {
+#pragma unroll 1
+    for (int u = tid; u < ns * K; u += PMDI_NT) {
+      const PoolDev& pd = sp.pd[T.u_ks[u] & 0xff];
+      const int c1 = T.u_c1[u], c2 = T.u_c2[u];
+      if (c2 >= 0) __stcg(pd.chosen + (size_t)b3 * pd.cap + c2, 0);
+      if (c1 >= 0) __stcg(pd.chosen + (size_t)z3 * pd.cap + c1, 0);
+    }
+  } else if (e >= 0) {
+#pragma unroll 1
+    for (int i = e + GE * tid; i < sm.cnt; i += GE * PMDI_NT) {  // the entries this CTA owns
+      const int4 en = spec_entry(sp, T, e, sm.lpar, i);
+      const PoolDev& pd = sp.pd[(unsigned)en.x >> SPEC_KSHIFT];
+      __stcg(pd.refcnt + (size_t)parn * pd.cap + (en.x & SPEC_VMASK), 0);
+    }
+  }
+  if (!spec_gsync(sp, sm)) return false;
+  // the recount: labels of one warp that refer to the same row are counted by one atomic
+#pragma unroll 1
+  for (int k = 0; k < K; ++k) {
+    const PoolDev& pd = sp.pd[k];
+    const int empty = pd.cap - 1;
+    const int* rm_new = pd.rowmap + (size_t)((ev + 1) & 1) * P * N;
+    int* rc_new = pd.refcnt + (size_t)parn * pd.cap;
+#pragma unroll 1
+    for (long long ib = (gt >> 5) << 5; ib < (long long)P * N; ib += GT) {
+      const long long i = ib + lane;
+      const int r = i < (long long)P * N ? ldcg_i32(rm_new + i) : empty;
+      const unsigned same = __match_any_sync(FULL, r);
+      if (r != empty && lane == __ffs(same) - 1) atomicAdd(rc_new + r, __popc(same));
+    }
+  }
+  if (is_p) spec_load_units<GRP>(sp, sm, T, ns);  // the new row maps are complete
+  if (!spec_gsync(sp, sm)) return false;
+  RS_MARK(5)
+  if (!is_p && e >= 0) {
+    const int lo = sm.lpar, ln = lo ^ 1, n_old = sm.cnt;
+    const bool ids2 = st + 2 < sp.steps;  // E'(st+2) ran: the ids of step st+2 are handed out
+    int nb = 0;
+#pragma unroll 1
+    for (int base = 0; base < n_old; base += PMDI_NT) {
+      const int i = base + tid;
+      int4 en = make_int4(0, 0, 0, 0);
+      int rc = 0;
+      if (i < n_old) {
+        en = spec_entry(sp, T, e, lo, i);
+        const int k = (unsigned)en.x >> SPEC_KSHIFT, v = en.x & SPEC_VMASK, c = en.y;
+        const PoolDev& pd = sp.pd[k];
+        rc = ldcg_i32(pd.refcnt + (size_t)parn * pd.cap + v);
+        if (rc == 0 && (i % GE) == e) {  // dead: the row, its child, their ids of step st+2
+          spec_free_id(sp, T, k, v);
+          spec_free_id(sp, T, k, c);
+          if (ids2) {
+            spec_free_id(sp, T, k, ldcg_info(pd.info + (size_t)(parn ^ 1) * pd.cap + v).z);
+            spec_free_id(sp, T, k, ldcg_info(pd.info + (size_t)(parn ^ 1) * pd.cap + c).z);
+          }
+        }
+      }
+      const unsigned keep = __ballot_sync(FULL, rc > 0);
+      if (lane == 0) sm.wsum[warp] = __popc(keep);
+      __syncthreads();
+      int wpre = 0, tot = 0;
+#pragma unroll
+      for (int w = 0; w < PMDI_NW; ++w) {
+        const int x = sm.wsum[w];
+        if (w < warp) wpre += x;
+        tot += x;
+      }
+      if (rc > 0) spec_set_entry(sp, T, e, ln, nb + wpre + __popc(keep & ((1u << lane) - 1u)), en);
+      nb += tot;
+      __syncthreads();
+    }
+    // rows evaluated ahead for step st+1 that this resampling killed
+    if (e == 0 && tid == 0) atomicAdd((unsigned long long*)&sp.counters[4], (unsigned long long)(n_old - nb));
+    if (tid < K) sm.kc[tid] = 0;
+    if (tid == 0) { sm.cnt = nb; sm.lpar = ln; }
+    spec_load_empty_next(sp, sm, parn);
+  }
+  RS_MARK(7)
+#undef RS_MARK
+  __syncthreads();
+  return !sm.fail;
+}
+
+// Pool accounting at the end of a sweep on one GPU (the instrumented kernel): every row id of a dataset is in exactly
+// one place - on the free stack, in one E-CTA's free-id cache, a row of the live-row list or that row's child of the
+// last step (the list after the fix of step steps-2: the last step's outcome is never fixed, the final resampling
+// leaves the list as it is), the empty row or its child of the last step.  Each place counts its ids into the mark
+// array (zero since the set-up: on one GPU nothing else writes it); a row counted twice was handed out or freed twice,
+// a row counted never has leaked.  Either ends the sweep with error 97.
+template <bool GRP>
+__device__ __noinline__ bool spec_check_pool(const SweepParams& sp, SpecSmem& sm, const SpecTables& T, int e) {
+  const int K = sp.K, GE = sp.G - sp.GP - 1, tid = threadIdx.x;
+  const long long gt = (long long)spec_cta<GRP>() * PMDI_NT + tid, GT = (long long)sp.G * PMDI_NT;
+  auto count = [&](const PoolDev& pd, int id) {
+    if (id >= 0 && id < pd.cap) atomicAdd(pd.mark + id, 1);
+    else { atomicExch(sp.err, 97); sm.fail = 1; }
+  };
+  if (!spec_gsync(sp, sm)) return false;  // every push and pop of the sweep is done
+#pragma unroll 1
+  for (int k = 0; k < K; ++k) {
+    const PoolDev& pd = sp.pd[k];
+    const int h = ldcg_i32(pd.ctr + 1);
+#pragma unroll 1
+    for (long long s = gt; s < h; s += GT) count(pd, ldcg_i32(pd.freelist + s));
+  }
+  if (e >= 0) {
+#pragma unroll 1
+    for (int k = 0; k < K; ++k)
+#pragma unroll 1
+      for (int i = tid; i < T.fc_top[k]; i += PMDI_NT) count(sp.pd[k], T.fc_s[k * SPEC_FC + i]);
+#pragma unroll 1
+    for (int i = e + GE * tid; i < sm.cnt; i += GE * PMDI_NT) {  // the entries this CTA owns
+      const int4 en = spec_entry(sp, T, e, sm.lpar, i);
+      const PoolDev& pd = sp.pd[(unsigned)en.x >> SPEC_KSHIFT];
+      count(pd, en.x & SPEC_VMASK);
+      count(pd, en.y);
+    }
+    if (e == 0 && tid < K) { count(sp.pd[tid], sp.pd[tid].cap - 1); count(sp.pd[tid], sm.b_next[tid]); }
+  }
+  if (!spec_gsync(sp, sm)) return false;
+#pragma unroll 1
+  for (int k = 0; k < K; ++k) {
+    const PoolDev& pd = sp.pd[k];
+#pragma unroll 1
+    for (long long r = gt; r < pd.cap; r += GT)
+      if (ldcg_i32(pd.mark + r) != 1) { atomicExch(sp.err, 97); sm.fail = 1; }
+  }
+  __syncthreads();
+  return !sm.fail;
+}
+
 template <bool DBG, bool GRP>
 __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem& sm, unsigned char* smem_raw, int* s_tmp) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1217,6 +1418,9 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
   else { __syncthreads(); if (!spec_wait_decision(sp, sm, steps - 1)) return; }
   const int final_res = sm.res_flag;
   if (final_res && !spec_resample<GRP>(sp, sm, T, ns, steps - 1, s_tmp, is_p, is_d ? -1 : e)) return;
+  if constexpr (DBG) {
+    if (sp.R == 1 && !spec_check_pool<GRP>(sp, sm, T, (is_p || is_d) ? -1 : e)) return;
+  }
   if (tid < K) {
     atomicAdd(sp.rows_eval + tid, (unsigned long long)sm.rows_eval[tid]);
     atomicAdd(sp.rows_ref + tid, (unsigned long long)sm.rows_ref[tid]);
