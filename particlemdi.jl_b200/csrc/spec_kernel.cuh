@@ -1390,7 +1390,10 @@ __device__ __forceinline__ void spec_sweep_body(const SweepParams& sp, SpecSmem&
 #endif
       if (t > 0) spec_fix<DBG>(sp, sm, T, e, t - 1);
       else spec_refresh_children(sp, sm, T, e);
-      // the distinct clusters the reference evaluates at step t (src/pmdi.jl:218-220): the list and the empty one
+      // the distinct clusters the reference evaluates at step t (src/pmdi.jl:218-220): the list and the empty one.
+      // The empty one is counted at every step, as k_empty_lp evaluates it for every step; the reference stops
+      // evaluating it once a resampling leaves no particle with an empty label (its pool renumbering,
+      // src/pmdi.jl:329-339, then drops it), so from there on this count has one row more per step and dataset.
       if (e == 0 && tid < K) { sm.rows_eval[tid] += (unsigned)sm.kc[tid] + 1u; sm.kc[tid] = 0; }  // the next fix counts afresh
       PHASE_MARK(3)
       SWEEP_TRACE(t, 51)

@@ -14,7 +14,9 @@ pytestmark = pytest.mark.gpu
 RTOL = 1e-5  # north_star tolerance for floating-point outputs
 
 
-ENGINES = ["pool", "dense"]  # copy-on-write pool (default) and the dense form, selected by PMDI_ENGINE
+# the speculative engine (the default for K <= 4), the copy-on-write pool (the default above) and the dense form,
+# selected by PMDI_ENGINE
+ENGINES = ["spec", "pool", "dense"]
 
 
 def _run_both(pr, tapes=None, seed=11, it=3, lw0=0.0, flags=None, engine="pool"):
@@ -92,26 +94,26 @@ def test_sweep_with_feature_flags(engine):
     _assert_parity(pr, ref, got)
 
 
-@pytest.mark.parametrize("engine", ENGINES)
+@pytest.mark.parametrize("engine", ["pool", "dense"])
 @pytest.mark.parametrize("name", ["gauss_wide", "mixed_k3", "mixed_k2_manyP"])
 @pytest.mark.parametrize("qb", ["1", "8"])
 def test_parity_for_other_item_sizes(name, qb, engine, monkeypatch):
     """The number of 256-feature blocks per work item is chosen per workload / per step (whole rows when
-    there are many rows per warp); parity must not depend on it."""
+    there are many rows per warp); parity must not depend on it.  Only the dense engine's work items read
+    PMDI_QB, so the spec engine is left out here: the other tests of this file run it on these cases."""
     monkeypatch.setenv("PMDI_QB", qb)
     pr = problem(**CASES[name], seed=5)
     ref, got = _run_both(pr, lw0=1.0, engine=engine)
     _assert_parity(pr, ref, got)
 
 
-@pytest.mark.parametrize("name", ["gauss_iris_shape", "mixed_k3", "mixed_k2_manyP", "gauss_N40"])
-def test_pool_evaluates_each_distinct_cluster_once(name):
-    """The copy-on-write pool performs exactly the reference's calc_logprob calls: one per distinct
-    cluster per (observation, dataset) - the oracle's de-duplicated mode counts them the way
-    src/__pmdi.jl:187 does (n_operations)."""
+DISTINCT = ["gauss_iris_shape", "mixed_k3", "mixed_k2_manyP", "gauss_N40"]
+
+
+def _assert_evaluates_each_distinct_cluster_once(name, engine):
     from oracle import oracle as orc
     pr = problem(**CASES[name], seed=7)
-    ref, got = _run_both(pr, lw0=1.0, engine="pool")
+    ref, got = _run_both(pr, lw0=1.0, engine=engine)
     _assert_parity(pr, ref, got)
     o = orc.Oracle(pr["data"], pr["types"], pr["N"], pr["P"])
     dd = o.sweep(pr["s"], pr["order"], pr["n1"], pr["Pi"], pr["phi"], mode=orc.MODE_DEDUP, logweight_init=1.0,
@@ -121,6 +123,21 @@ def test_pool_evaluates_each_distinct_cluster_once(name):
     # evaluated once more than in the reference; the kernel counts them
     assert sum(got["rows_evaluated"]) - got["rows_evaluated_ahead"] == dd["n_ops"]
     assert sum(got["rows_referenced"]) >= sum(got["rows_evaluated"]) - pr["K"] * (pr["n"] - pr["n1"] + 1)
+
+
+@pytest.mark.parametrize("name", DISTINCT)
+def test_pool_evaluates_each_distinct_cluster_once(name):
+    """The copy-on-write pool performs exactly the reference's calc_logprob calls: one per distinct
+    cluster per (observation, dataset) - the oracle's de-duplicated mode counts them the way
+    src/__pmdi.jl:187 does (n_operations)."""
+    _assert_evaluates_each_distinct_cluster_once(name, "pool")
+
+
+@pytest.mark.parametrize("name", DISTINCT)
+def test_spec_evaluates_each_distinct_cluster_once(name):
+    """The same count for the speculative engine, whose evaluation CTAs walk the live-row list one
+    observation ahead of the resampling decision."""
+    _assert_evaluates_each_distinct_cluster_once(name, "spec")
 
 
 def test_sstar_compat_flag():
