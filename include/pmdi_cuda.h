@@ -345,8 +345,26 @@ int pmdi_psm_get(pmdi_ctx* ctx, double* out);
  *                           on ties; partition_out: its n_obs labels 1..N.  Any output may be NULL.
  *   pmdi_summary_agreement  chains >= 2: for every pair of chains a < b (row-major) and dataset k, out[pair * K + k] =
  *                           max (max_out) and mean (mean_out) over i < j of |PSM_a(i,j) - PSM_b(i,j)|.
+ *   pmdi_summary_hclust     exact agglomerative clustering of the pooled PSM of dataset k (k = -1: Overall), the
+ *                           reference's get_consensus_allocations tree (consensus_map.jl:92-105) with the linkage
+ *                           named: PMDI_LINK_SINGLE, _COMPLETE or _AVERAGE (UPGMA).  With A_ij the pooled pair count
+ *                           (summed over the datasets for Overall) and U = rows (K * rows for Overall), the
+ *                           dissimilarity of a pair is 1 - A_ij / U; a cluster pair's similarity is s / p with s the max
+ *                           (single), min (complete) or sum (average) of A_ij over its pairs and p = 1 or |X| |Y|
+ *                           (average).  Each merge takes the largest s / p, compared exactly; among equals, the
+ *                           lexicographically smallest (smaller, larger) pair of representatives (a cluster's smallest
+ *                           observation index).  Z_out: the (n_obs - 1) x 4 row-major scipy linkage matrix, [smaller id,
+ *                           larger id, height, size], leaves 0..n_obs-1 and merge m creating n_obs + m, height =
+ *                           (double)(p U - s) / (double)(p U).  rescans_out (may be NULL): the rows whose best partner
+ *                           had to be found again by a full scan, summed over the merges.  Refuses, before allocating,
+ *                           working storage that does not fit in free device memory (about 8 n_obs^2 bytes for
+ *                           average, 4 n_obs^2 otherwise); the message states the bytes needed.  n_obs = 1: nothing is
+ *                           written.  DESIGN.md §16.
  *   pmdi_summary_destroy    waits for the summary's work and frees everything.
  */
+#define PMDI_LINK_SINGLE   0
+#define PMDI_LINK_COMPLETE 1
+#define PMDI_LINK_AVERAGE  2
 typedef struct pmdi_summary pmdi_summary;
 int pmdi_summary_create(pmdi_summary** out, int32_t device, int32_t K, int64_t n_obs, int32_t N, int32_t chains);
 int pmdi_summary_add(pmdi_summary* summary, int32_t chain, const int64_t* s, int64_t rows);
@@ -355,6 +373,8 @@ int pmdi_summary_psm(pmdi_summary* summary, int32_t chain, int32_t k, void* out,
 int pmdi_summary_ls(pmdi_summary* summary, int32_t k, double* loss_out, int32_t* best_chain, int64_t* best_row,
                     int64_t* partition_out);
 int pmdi_summary_agreement(pmdi_summary* summary, double* max_out, double* mean_out);
+int pmdi_summary_hclust(pmdi_summary* summary, int32_t k, int32_t linkage, double* Z_out /* (n_obs-1)*4 */,
+                        int64_t* rescans_out /* may be NULL */);
 int pmdi_summary_destroy(pmdi_summary* summary);
 /* Host only (no device needed): the allocation columns of `rows` CSV rows of pmdi()'s output (header excluded), one
  * row per line.  Each row's first `skip` columns are skipped, then `count` labels are read, written as integers

@@ -503,6 +503,10 @@ def read_chains(outputFiles, burnin=0, thin=1):
 
 def _summary_of(outputFiles, burnin, thin, device):
     chains, _ = read_chains(outputFiles, burnin, thin)
+    return _summary_of_chains(chains, device)
+
+
+def _summary_of_chains(chains, device):
     rows, n_obs, K = chains[0].shape
     if any(c.shape[0] == 0 for c in chains):
         raise ValueError("a chain keeps no rows after burnin / thin")
@@ -536,6 +540,49 @@ def chain_agreement(outputFiles, burnin=0, thin=1, device=0):
     two arrays of shape (C (C - 1) / 2, K)."""
     with _summary_of(outputFiles, burnin, thin, device) as S:
         return S.agreement()
+
+
+def cut_tree(Z, n_clusters):
+    """Labels 1..n_clusters of the n observations of scipy linkage matrix Z ((n - 1) x 4) cut into n_clusters: the
+    last n_clusters - 1 merges (rows of Z) undone, the clusters numbered in order of their smallest observation
+    index.  This is ``scipy.cluster.hierarchy.cut_tree(Z, n_clusters).ravel() + 1`` whenever the cut falls between
+    two different heights; scipy takes merges of equal height in an order of its own, not by their row in Z."""
+    Z = np.asarray(Z, dtype=np.float64)
+    if Z.ndim != 2 or Z.shape[1] != 4:
+        raise ValueError(f"Z must be (n - 1, 4), not {Z.shape}")
+    n = Z.shape[0] + 1
+    if not 1 <= int(n_clusters) <= n:
+        raise ValueError(f"n_clusters {n_clusters} outside 1..{n}")
+    rep = np.arange(2 * n - 1)  # smallest observation of every cluster id
+    parent = np.arange(n)
+    for m in range(n - int(n_clusters)):
+        u, v = rep[int(Z[m, 0])], rep[int(Z[m, 1])]
+        lo, hi = min(u, v), max(u, v)
+        parent[hi] = lo
+        rep[n + m] = lo
+    while True:  # pointer jumping to the roots, each the smallest observation of its cluster
+        up = parent[parent]
+        if (up == parent).all():
+            break
+        parent = up
+    return np.unique(parent, return_inverse=True)[1].astype(np.int64) + 1
+
+
+def consensus_allocations(outputFiles, n_clusters, linkage, dataset=None, burnin=0, thin=1, device=0):
+    """The reference's ``get_consensus_allocations(psm, k)`` (consensus_map.jl:92-105) over one CSV file or the files
+    of several chains, pooled: the PSM of dataset ``dataset`` (0-based; None: Overall) clustered on the GPU with the
+    named ``linkage`` ("single", "complete" or "average"; ``PosteriorSummary.hclust``), the tree cut into
+    ``n_clusters``.  Returns n_obs labels in 1..n_clusters, numbered in order of their smallest observation."""
+    if linkage not in capi.LINKAGES:
+        raise ValueError(f"linkage is one of {sorted(capi.LINKAGES)}, not {linkage!r}")
+    chains, _ = read_chains(outputFiles, burnin, thin)
+    _, n_obs, K = chains[0].shape
+    if not 1 <= int(n_clusters) <= n_obs:
+        raise ValueError(f"n_clusters {n_clusters} outside 1..{n_obs}")
+    if dataset is not None and not 0 <= int(dataset) < K:
+        raise ValueError(f"dataset {dataset} outside 0..{K - 1}")
+    with _summary_of_chains(chains, device) as S:
+        return cut_tree(S.hclust(dataset, linkage=linkage), n_clusters)
 
 
 def posterior_similarity(alloc):
