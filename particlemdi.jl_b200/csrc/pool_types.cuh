@@ -28,7 +28,7 @@
       const double dd = __dadd_rn(x.C, -mu[i].C);                                                    \
       bt[i].C = __dadd_rn(bt[i].C, div_const(__dmul_rn(c1, __dmul_rn(dd, dd)), c2, r2));             \
       mu[i].C = div_const(sm[i].C, c3, r3);                                                          \
-      ln[i].C = div_const(pm_div(c4, __dmul_rn(bt[i].C, c5)), c6, r6);                               \
+      ln[i].C = div_const(div_rn(c4, __dmul_rn(bt[i].C, c5)), c6, r6);                               \
       pl *= ln[i].C;                                                                                 \
       const double d_ = y.C - mu[i].C;                                                               \
       pd *= fma(d_ * d_, ln[i].C, 1.0);                                                              \
@@ -50,6 +50,7 @@ __device__ __noinline__ double gauss_block(const double* s_sum, const double* s_
     c6 = __dadd_rn(nn, 1.0);
     r2 = __drcp_rn(c2); r3 = __drcp_rn(c3); r6 = __drcp_rn(c6);
   }
+  const double aux = mode != 1 ? ldcg_f64(s_aux) : 0.0;  // in flight with the statistics
   double pl = 1.0, pd = 1.0, ps = 1.0;
 #pragma unroll 1
   for (int h = 0; h < nit; h += 2) {
@@ -89,7 +90,7 @@ __device__ __noinline__ double gauss_block(const double* s_sum, const double* s_
     es += __shfl_xor_sync(FULL, es, o);
   }
   double vs = 0.0;
-  if (mode != 1) vs = ldcg_f64(s_aux) - (0.5 * (double)n + 1.0) * es;
+  if (mode != 1) vs = aux - (0.5 * (double)n + 1.0) * es;
   if (mode == 0) return vs;
   if ((threadIdx.x & 31) == 0) *d_aux = a;
   *v_src = vs;

@@ -657,7 +657,7 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
   for (int j0 = e; j0 < total; j0 += GE * rpc, buf ^= 1) {
     const int j = j0 + sub * GE;
     bool active = sub < rpc && j < total;
-    int k = 0, v = 0, c = 0, nc = 0;
+    int k = 0, v = 0, c = 0, nc = 0, id = 0;
     double rcv = 0.0;
     if (active) {
       if (j < n_list) {
@@ -724,6 +724,7 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
         }
       }
     }
+    if (active && wj == 0 && lane < 2 && (mode || lane == 1)) id = spec_pop_id(sp, sm, T, k);  // while the other warps finish
     SWEEP_TRACE(st - 1, 64)
     __syncthreads();
     SWEEP_TRACE(st - 1, 65)
@@ -731,12 +732,17 @@ __device__ __noinline__ void spec_eval(const SweepParams& sp, SpecSmem& sm, cons
       const DsDev& ds = sp.ds[k];
       const PoolDev& pd = sp.pd[k];
       const int r0 = ds.J <= jq ? sub * jq : 0;
-      int id = 0;
       double lv = rcv;
       if (lane < 2 && (mode || lane == 1)) {
 #pragma unroll 1
-        for (int jb = 0; jb < ds.J; ++jb) lv += sm.red[buf][lane][r0 + jb];
-        id = spec_pop_id(sp, sm, T, k);  // the id of the next child; its cluster size is known now
+        for (int j0 = 0; j0 < ds.J; j0 += 16) {  // independent loads, then the sum in block order
+          double pv[16];
+#pragma unroll
+          for (int u = 0; u < 16; ++u) pv[u] = j0 + u < ds.J ? sm.red[buf][lane][r0 + j0 + u] : 0.0;
+#pragma unroll
+          for (int u = 0; u < 16; ++u)
+            if (j0 + u < ds.J) lv += pv[u];
+        }
         SCHECK(id >= 0 && id < pd.cap - 1 && id != v && id != c, 92)
         __stcg(ds.n + id, nc + 2 - lane);
       }
